@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- rendered rays/sec of one NICE-SLAM tracking iteration (fwd + loss + bwd) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 Workload (BASELINE.json metric "rendered rays/sec (200px x 48samp batch) ... ms/tracking-iter"): Replica room0 geometry,
@@ -18,6 +18,10 @@ caller reads the result).  The two host blocks can travel as copy-engine nodes (
 memory ("sm"), or with the result stored by the backward's last CTA ("sm_push"); all three are timed, checked to deliver identical bytes, and
 the fastest is reported (`e2e.ms_per_step_by_transport` keeps the three figures).  --impl reference times the reference algorithm's CPU path (oracle port, PyTorch CPU, all host
 threads) on the same batch.  Every timed quantity uses CUDA events on the launching stream, max over ranks.
+
+--dump-outputs DIR: after the timed steps, what the last timed step handed its caller is written as DIR/<name>.npy (float32 / float64, rank 0):
+one GPU: loss, d_c2w, depth, var, rgb, d_rays_o, d_rays_d of the 200-ray iteration; N > 1: the summed loss and d_c2w; --impl reference: loss
+and d_c2w.  The inputs are generated from fixed seeds, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -195,8 +199,10 @@ def run_reference(args):
         step()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        step()
+        loss, d_c2w = step()
     ms = (time.perf_counter() - t0) / args.steps * 1e3
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"loss": torch.tensor([loss], dtype=torch.float64), "d_c2w": d_c2w})
     value = n_rays / (ms * 1e-3)
     line = {"impl": "reference", "metric": METRIC, "value": value, "unit": "rays/s", "n_gpus": args.gpus, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": ms, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32",
@@ -637,6 +643,12 @@ def run_native(args):
         sampler.start()
     total_ms, t0, t1 = timed(step_dev, args.steps, max(args.warmup, 3), True)
     clocks = sampler.stop(t0, t1) if rank == 0 else None
+    if args.dump_outputs and rank == 0:                            # before the loops below overwrite the context's buffers
+        if sharded is None:
+            dump_outputs(args.dump_outputs, {"loss": ctx.loss, "d_c2w": ctx.d_c2w, "depth": ctx.depth, "var": ctx.var, "rgb": ctx.rgb,
+                                             "d_rays_o": ctx.d_rays_o, "d_rays_d": ctx.d_rays_d})
+        else:
+            dump_outputs(args.dump_outputs, {"loss": sharded.packed[:1], "d_c2w": sharded.packed[1:].view(3, 4)})
     # dominant kernel (render_bwd_kernel): events recorded by the library around its launch, averaged over a short loop
     bwd_ms = []
     ctx.time_backward(True)
@@ -755,6 +767,15 @@ def shutdown(world):
         os._exit(0)
 
 
+def dump_outputs(dirname, arrays):
+    """{name: tensor} -> dirname/<name>.npy, float64 tensors as float64, everything else as float32."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach().cpu()
+        np.save(os.path.join(dirname, name + ".npy"), t.numpy().astype(np.float64 if t.dtype == torch.float64 else np.float32))
+
+
 _REAL_STDOUT = None
 
 
@@ -778,7 +799,11 @@ def main():
     ap.add_argument("--steps", type=int, default=None)
     ap.add_argument("--warmup", type=int, default=None)
     ap.add_argument("--impl", default="native", choices=["native", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (see the module docstring)")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         args.steps = 30 if args.steps is None else args.steps
         args.warmup = 3 if args.warmup is None else args.warmup

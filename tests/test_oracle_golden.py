@@ -18,6 +18,18 @@ TOL = 1e-4      # north_star tolerance (rel) -- the oracles actually agree to ~1
 # dominated by f32 rounding of (1 - alpha); the reference's own f32 run differs from its f64 evaluation by 8e-4 there
 # (measured, DESIGN.md "tolerances"), so those tensors get a noise-floor tolerance instead of 1e-4.
 TOL_SATURATED = 3e-3
+# The fixtures hold the reference's float32 bits as PyTorch computed them with 8 CPU threads.  MKL's sgemm splits its sums by the
+# thread count, so any other count changes the bits: the bit-exact comparisons run on exactly 8 threads, whatever the machine's
+# core count.  (By default MKL runs at most one thread per physical core: this needs a machine with 8 cores or more.)
+FIXTURE_THREADS = 8
+
+
+@pytest.fixture(autouse=True, scope="module")
+def fixture_thread_count():
+    n = torch.get_num_threads()
+    torch.set_num_threads(FIXTURE_THREADS)
+    yield
+    torch.set_num_threads(n)
 
 
 def dec_tol(variant, lvl):
