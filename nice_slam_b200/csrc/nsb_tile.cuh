@@ -14,7 +14,9 @@
 //     (TMA -> issuer) and empty (tcgen05.commit -> producer) mbarriers: three units of prefetch, no thread touches a weight;
 //   * activations ping-pong between two 32 KB operand buffers; warps publish a tile by fence.proxy.async + one mbarrier.arrive per warp
 //     (A_ready); thread 0 waits for the eight arrivals, issues the group's MMAs and commits to the buffer's `done` barrier -- there is no
-//     __syncthreads in the chain, and the gather / embedding of tile n+1 overlaps the MMAs of tile n.
+//     __syncthreads in the chain, and the gather / embedding of tile n+1 overlaps the MMAs of tile n.  Operands that the epilogue threads
+//     produce row by row (the forward's hidden-layer inputs, the hi parts of the backward's G / DU) go to TENSOR memory instead
+//     (tcgen05.st, tcgen05.wait::st before the arrival): shared-memory operand reads are what bound the MMA groups.
 // Shared memory: 64 KB activations + 40 KB ring + 6 KB headers + < 6 KB state <= 113 KB, TMEM 256 columns -> two CTAs per SM, i.e. two
 // tiles in flight per SM with the hardware interleaving their (latency-bound) chains.
 //
@@ -75,6 +77,12 @@ __device__ __forceinline__ void tmem_ld16(uint32_t taddr, float (&v)[16]) {
   asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 #pragma unroll
   for (int j = 0; j < 16; j++) v[j] = __uint_as_float(r[j]);
+}
+// this thread's 16 columns of its lane (row); ordered before a tcgen05.mma of another thread by tcgen05.wait::st + publish_tmem
+__device__ __forceinline__ void tmem_st16(uint32_t taddr, const float (&v)[16]) {
+  asm volatile("tcgen05.st.sync.aligned.32x32b.x16.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16};"
+               ::"r"(taddr), "f"(v[0]), "f"(v[1]), "f"(v[2]), "f"(v[3]), "f"(v[4]), "f"(v[5]), "f"(v[6]), "f"(v[7]),
+                 "f"(v[8]), "f"(v[9]), "f"(v[10]), "f"(v[11]), "f"(v[12]), "f"(v[13]), "f"(v[14]), "f"(v[15]) : "memory");
 }
 
 // ---- shared memory -------------------------------------------------------------------------------------------------------------
@@ -222,6 +230,36 @@ __device__ __forceinline__ void mma_unit(Issuer& I, const TileSmem& t, uint32_t 
   I.issued++;
   acc = 1u;
 }
+// The same unit (same three products, same order, same accumulator) with the A operand in TENSOR MEMORY: one row per lane, k-step ks at
+// column +8 ks.  A hi is read from columns a_hi; A lo from columns a_lo, or -- a_lo_s != nullptr -- from the canonical shared-memory tile a_lo_s.
+// Every N <= 64 MMA re-reads its whole [128 x 8] A slice, and the shared-memory operand reads are what bound the tensor pipe here
+// (probe_tmem_a_unit.cu); tensor-memory A takes those bytes off shared memory.
+__device__ __forceinline__ void mma_tf32_ta(uint32_t d_tmem, uint32_t a_tmem, uint64_t db, uint32_t idesc, uint32_t accumulate) {
+  asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
+               "tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1], %2, %3, p;\n\t}"
+               ::"r"(d_tmem), "r"(a_tmem), "l"(db), "r"(idesc), "r"(accumulate) : "memory");
+}
+template <int KSTEPS>
+__device__ __forceinline__ void mma_unit_ta(Issuer& I, const TileSmem& t, uint32_t d_tmem, uint32_t a_hi, uint32_t a_lo, const float* a_lo_s, const float* b, int N, int KB,
+                                            uint32_t& acc, uint64_t* done = nullptr) {
+  const uint32_t idesc = tc::make_idesc(TM, N);
+  const uint64_t bh = tc::make_desc(b, 128u, (uint32_t)(KB >> 2) * 128u);
+  const uint64_t bl = bh + (uint64_t)((N * KB * 4) >> 4);
+  const uint64_t al = a_lo_s != nullptr ? tc::make_desc(a_lo_s, 128u, 8u * 128u) : 0ull;
+  if (elect_one()) {
+#pragma unroll
+    for (int ks = 0; ks < KSTEPS; ks++) {
+      if (a_lo_s != nullptr) tc::mma_tf32(d_tmem, al + 16u * ks, bh + 16u * ks, idesc, ks == 0 ? acc : 1u);
+      else mma_tf32_ta(d_tmem, a_lo + 8u * ks, bh + 16u * ks, idesc, ks == 0 ? acc : 1u);
+      mma_tf32_ta(d_tmem, a_hi + 8u * ks, bl + 16u * ks, idesc, 1u);
+      mma_tf32_ta(d_tmem, a_hi + 8u * ks, bh + 16u * ks, idesc, 1u);
+    }
+    tc::mma_commit(t.bars + B_EMPTY + (I.issued & (kSlots - 1)));
+    if (done != nullptr) tc::mma_commit(done);
+  }
+  I.issued++;
+  acc = 1u;
+}
 
 // ---- FP16 hi|lo forward (option fwd_f16) ------------------------------------------------------------------------------------------------------
 // x = hi + lo with hi = fp16(x), lo = fp16(x - hi): 22 significant bits for |x| in [2^-3, 65504], an absolute error <= 2^-25 below (lo goes
@@ -295,6 +333,25 @@ __device__ __forceinline__ void publish(const TileSmem& t, int b) {
   fence_proxy_async(); tc::tc_fence_before();
   __syncwarp();                                                 // one arrival per warp (256 arrivals on one barrier word serialise)
   if ((threadIdx.x & 31) == 0) mbar_arrive(t.bars + B_AREADY + b);
+}
+// the same for operands of this thread written to tensor memory (and, SMEM, also to shared memory)
+template <bool SMEM>
+__device__ __forceinline__ void publish_tmem(const TileSmem& t, int b) {
+  asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+  if (SMEM) fence_proxy_async();
+  tc::tc_fence_before();
+  __syncwarp();
+  if ((threadIdx.x & 31) == 0) mbar_arrive(t.bars + B_AREADY + b);
+}
+// 3xTF32 split of this thread's 16 features (as tc::put4): hi = the bits the tensor core reads, lo = v - hi (exact)
+__device__ __forceinline__ void split16(const float (&v)[kCW], float (&hi)[kCW], float (&lo)[kCW]) {
+#pragma unroll
+  for (int j = 0; j < kCW; j++) { hi[j] = tc::to_tf32(v[j]); lo[j] = v[j] - hi[j]; }
+}
+// 16 features (column half cg) of row r -> one canonical [128 x 32] tile
+__device__ __forceinline__ void put16(float* tile, int r, int cg, const float (&v)[kCW]) {
+#pragma unroll
+  for (int k = 0; k < kKQ; k++) *reinterpret_cast<float4*>(tile + tc::canon_q(r, kKQ * cg + k, 32)) = make_float4(v[4 * k], v[4 * k + 1], v[4 * k + 2], v[4 * k + 3]);
 }
 __device__ __forceinline__ void wait_group(const TileSmem& t, uint32_t m) {      // MMAs of operand group m (and all earlier ones) have completed
   mbar_wait_b(t.bars + B_DONE + (m & 1u), (m >> 1) & 1u);
@@ -387,7 +444,11 @@ __device__ __forceinline__ void embed_tile(float* e_hi, const float* B, const fl
 }
 
 // ---- forward: what the issuing thread (thread 0) does after the CTA published operand group I.g --------------------------------------------
-// TMEM: D1 = [0,32), D3 = [32,64) (layer 3; its skip part is accumulated while the embedding blocks are live), D2 = [64,224) (fc_c of the five layers)
+// TMEM: D1 = [0,32), D3 = [32,64) (layer 3; its skip part is accumulated while the embedding blocks are live), D2 = [64,224) (fc_c of the five layers),
+// [224,256) = A lo of the hidden layers.  The A operand of layer i+1 (the ReLU output of layer i) never goes through shared memory (3xTF32 path):
+// its hi part overwrites D2 slice i, whose last reader is epilogue i itself (the same lanes and columns, just before), its lo part goes to
+// [224,256), whose last reader (layer i's MMAs) has completed when epilogue i starts.
+constexpr uint32_t kFwdALo = 224u;
 template <bool H16 = false>
 __device__ __forceinline__ void issue_fc(Issuer& I, const TileSmem& t, uint32_t tmem, int half) {      // C tile `half` -> D2 += C * Wc^T (four K = 8 units)
   const int b = I.g & 1;
@@ -431,7 +492,7 @@ __device__ __forceinline__ void issue_h(Issuer& I, const TileSmem& t, uint32_t t
   const float* w = issuer_unit(I, t);
   uint32_t acc = i == 3 ? 1u : 0u;
   if (H16) mma_unit_h<2>(I, t, i == 3 ? tmem + 32u : tmem, t.a[b], 0, w, 32, 32, acc, t.bars + B_DONE + b);
-  else mma_unit<4>(I, t, i == 3 ? tmem + 32u : tmem, t.a[b], 0, w, 32, 32, 0, acc, t.bars + B_DONE + b);
+  else mma_unit_ta<4>(I, t, i == 3 ? tmem + 32u : tmem, tmem + 64u + 32u * (i - 1), tmem + kFwdALo, nullptr, w, 32, 32, acc, t.bars + B_DONE + b);
   I.g++;
 }
 
@@ -497,14 +558,16 @@ __device__ __forceinline__ void epi_forward(const KParams& P, const TileSmem& t,
       for (int k = 0; k < kKQ; k++) __stcg(reinterpret_cast<float4*>(acts + i * 32 + 4 * k), make_float4(h[4 * k], h[4 * k + 1], h[4 * k + 2], h[4 * k + 3]));
     }
     if (i == 4) break;
-    float* h_hi = t.a[n & 1];
-    if (H16) put16_h(h_hi, row, cg, h);
+    if (H16) put16_h(t.a[n & 1], row, cg, h);
     else {
-#pragma unroll
-      for (int k = 0; k < kKQ; k++) tc::put4(h_hi, h_hi + TM * 32, row, kKQ * cg + k, 32, make_float4(h[4 * k], h[4 * k + 1], h[4 * k + 2], h[4 * k + 3]));
+      float hi[kCW], lo[kCW];
+      split16(h, hi, lo);
+      tmem_st16(d2 + 32u * i, hi);
+      tmem_st16(tmem + kFwdALo + my, lo);
     }
     NSB_PH(8);
-    publish(t, n & 1); n++;
+    if (H16) publish(t, n & 1); else publish_tmem<false>(t, n & 1);
+    n++;
     if (t0) issue_h<H16>(I, t, tmem, i + 1);
     NSB_PH(9);
   }
@@ -666,27 +729,27 @@ __device__ __forceinline__ float warp_colsum16(const float (&v)[kCW], int lane) 
 __device__ __forceinline__ int colsum_col(int lane) { return ((lane >> 4) & 1) * 8 + ((lane >> 3) & 1) * 4 + ((lane >> 2) & 1) * 2 + ((lane >> 1) & 1); }
 
 // ---- backward (input gradients): what the issuing thread does after the CTA published layer i's operands (G in a[0], DU in a[1]) ---------------
-// TMEM: D1 = [0,32) (g of the next layer), DC = [32,96) (dL/dc), DF = [96,192) (dL/d first input).
+// TMEM: D1 = [0,32) (g of the next layer), DC = [32,96) (dL/dc), DF = [96,192) (dL/d first input).  render_bwd_tile_kernel: G hi = [192,224),
+// DU hi = [224,256) (their last readers, the previous layer's MMAs, have completed when the epilogue writes them); the lo parts stay in the lo
+// halves of a[0] / a[1].  render_bwd_wg_tile_kernel accumulates its weight gradients in [192,224) and keeps both operands in shared memory.
+constexpr uint32_t kBwdGHi = 192u, kBwdDuHi = 224u;
+// one A operand of the layer's products: G (a[0]) or DU (a[1]); TA: hi in tensor memory at column a_hi, lo in shared memory
+template <bool TA>
+__device__ __forceinline__ void mma_unit_bwd(Issuer& I, const TileSmem& t, uint32_t d_tmem, const float* a, uint32_t a_hi, const float* w, uint32_t acc) {
+  if (TA) mma_unit_ta<4>(I, t, d_tmem, a_hi, 0u, a + TM * 32, w, 32, 32, acc);
+  else mma_unit<4>(I, t, d_tmem, a, 0, w, 32, 32, 0, acc);
+}
+template <bool TA>
 __device__ __forceinline__ void issue_bwd_layer(Issuer& I, const TileSmem& t, uint32_t tmem, int lv, int i) {
   const bool xyz = lv != 0;
   const int cd = op_cd(lv), nfb = op_firstp(lv) / 32;
   issuer_wait_operands(I, t, 0, I.g & 1u);
-  if (xyz) for (int c2 = 0; c2 < cd / 32; c2++) {               // DC += G * Wc_i
-    const float* w = issuer_unit(I, t);
-    uint32_t acc = i == 4 ? 0u : 1u;
-    mma_unit<4>(I, t, tmem + 32u + 32u * c2, t.a[0], 0, w, 32, 32, 0, acc);
-  }
-  if (i >= 1) {                                                 // D1 = DU * W_i[:, hidden]
-    const float* w = issuer_unit(I, t);
-    uint32_t acc = 0u;
-    mma_unit<4>(I, t, tmem, t.a[1], 0, w, 32, 32, 0, acc);
-  }
+  if (xyz) for (int c2 = 0; c2 < cd / 32; c2++)                 // DC += G * Wc_i
+    mma_unit_bwd<TA>(I, t, tmem + 32u + 32u * c2, t.a[0], tmem + kBwdGHi, issuer_unit(I, t), i == 4 ? 0u : 1u);
+  if (i >= 1)                                                   // D1 = DU * W_i[:, hidden]
+    mma_unit_bwd<TA>(I, t, tmem, t.a[1], tmem + kBwdDuHi, issuer_unit(I, t), 0u);
   if (i == 3 || i == 0) {                                       // DF += DU * W_i[:, first input]
-    for (int fb = 0; fb < nfb; fb++) {
-      const float* w = issuer_unit(I, t);
-      uint32_t acc = i == 3 ? 0u : 1u;
-      mma_unit<4>(I, t, tmem + 96u + 32u * fb, t.a[1], 0, w, 32, 32, 0, acc);
-    }
+    for (int fb = 0; fb < nfb; fb++) mma_unit_bwd<TA>(I, t, tmem + 96u + 32u * fb, t.a[1], tmem + kBwdDuHi, issuer_unit(I, t), i == 3 ? 0u : 1u);
   }
   issuer_group_done(t, B_DONE);
   I.g++;
@@ -757,16 +820,29 @@ __device__ __forceinline__ void epi_backward(const KParams& P, const TileSmem& t
         atomicAdd(w->dpk + DW::o_b + 32 * i + col, sb); atomicAdd(w->dpk + DW::o_bc + 32 * i + col, sc);
       }
     }
+    if constexpr (WG) {
 #pragma unroll
-    for (int k = 0; k < kKQ; k++) {
-      if (xyz) tc::put4(g_hi, g_hi + TM * 32, row, kKQ * cg + k, 32, make_float4(g[4 * k], g[4 * k + 1], g[4 * k + 2], g[4 * k + 3]));
-      tc::put4(du_hi, du_hi + TM * 32, row, kKQ * cg + k, 32,
-               make_float4((m >> (4 * k)) & 1u ? g[4 * k] : 0.0f, (m >> (4 * k + 1)) & 1u ? g[4 * k + 1] : 0.0f,
-                           (m >> (4 * k + 2)) & 1u ? g[4 * k + 2] : 0.0f, (m >> (4 * k + 3)) & 1u ? g[4 * k + 3] : 0.0f));
+      for (int k = 0; k < kKQ; k++) {
+        if (xyz) tc::put4(g_hi, g_hi + TM * 32, row, kKQ * cg + k, 32, make_float4(g[4 * k], g[4 * k + 1], g[4 * k + 2], g[4 * k + 3]));
+        tc::put4(du_hi, du_hi + TM * 32, row, kKQ * cg + k, 32,
+                 make_float4((m >> (4 * k)) & 1u ? g[4 * k] : 0.0f, (m >> (4 * k + 1)) & 1u ? g[4 * k + 1] : 0.0f,
+                             (m >> (4 * k + 2)) & 1u ? g[4 * k + 2] : 0.0f, (m >> (4 * k + 3)) & 1u ? g[4 * k + 3] : 0.0f));
+      }
+      NSB_PH(22);
+      publish(t, 0);
+    } else {
+      float hi[kCW], lo[kCW];
+      if (xyz) { split16(g, hi, lo); tmem_st16(tmem + kBwdGHi + my, hi); put16(g_hi + TM * 32, row, cg, lo); }
+      float du[kCW];
+#pragma unroll
+      for (int j = 0; j < kCW; j++) du[j] = (m >> j) & 1u ? g[j] : 0.0f;
+      split16(du, hi, lo);
+      tmem_st16(tmem + kBwdDuHi + my, hi);
+      put16(du_hi + TM * 32, row, cg, lo);
+      NSB_PH(22);
+      publish_tmem<true>(t, 0);
     }
-    NSB_PH(22);
-    publish(t, 0);
-    if (threadIdx.x < 32) issue_bwd_layer(I, t, tmem, lv, i);
+    if (threadIdx.x < 32) issue_bwd_layer<!WG>(I, t, tmem, lv, i);
     NSB_PH(23);
     if constexpr (WG) {                                          // weight gradients of layer i (the chain's MMAs run meanwhile)
       if (i >= 1) {                                              // hidden input H_{i-1}
