@@ -78,9 +78,10 @@ size_t nsb_packed_decoder_floats(int level);
 
 int nsb_version(void);
 const char* nsb_last_error(void);
-/* Process-wide options.  "mlp_backend": 0 = auto (default: tcgen05 tile kernels), 1 = FP32-FMA decoders, 2 = tcgen05 round-1 ray-group
- * kernels, 3 = tcgen05 tile kernels (3xTF32, two CTAs per SM).  "split_model": 1 (default) = a tile's decoders are spread over CTAs only while
- * that beats one CTA per tile by wave efficiency, 0 = always for batches of <= 262144 points.  "wgrad_tc", "fwd_f16", "pdl", "small_rays": DESIGN.md. */
+/* Process-wide options.  "mlp_backend": 0 = auto (default: tcgen05 tile kernels, 3xTF32, two CTAs per SM; FP32-FMA decoders where
+ * n_samples + n_surface < 8), 1 = FP32-FMA decoders; other values return NSB_ERR_ARG.  "split_model": 1 (default) = a tile's decoders are
+ * spread over CTAs only while that beats one CTA per tile by wave efficiency, 0 = always for batches of <= 262144 points.  "wgrad_tc",
+ * "fwd_f16": DESIGN.md. */
 int nsb_set_option(const char* key, int value);
 
 /* Diagnostic: resident CTAs per SM of the tile-centric tensor-core kernels (2 = the design point: two tiles in flight per SM). */
@@ -131,9 +132,9 @@ typedef struct {
   int32_t* corner_idx;           /* optional [N,S,3]: (ix0,iy0,iz0) of the stage's finest occupancy grid */
   uint32_t* masks;               /* optional [N,S,15]: ReLU sign bits of the 5 layers of up to 3 decoders (stage order); when the
                                     backward pass receives them it does not recompute the forward (tensor-core backend only) */
-  void* split_workspace;         /* optional device scratch of nsb_split_workspace_bytes(N, S) bytes, ZEROED ONCE by the caller (the library
-                                    leaves it clean): lets small batches (N <= 256 rays, several decoders) run one CTA per decoder
-                                    and ray group instead of one CTA per ray group; NULL = never split */
+  void* split_workspace;         /* device scratch of nsb_split_workspace_bytes(N, S) bytes, ZEROED ONCE by the caller (the library
+                                    leaves it clean): ray completion counters and per-item partial results of the tile kernels, which
+                                    need it; the FP32-FMA kernels (S < 8, mlp_backend 1) do not read it */
   size_t split_workspace_bytes;
   float* acts;                   /* optional [N,S,5,32] float32: outputs of the five hidden layers of the decoder whose WEIGHT gradients the
                                     backward will be asked for (the colour decoder in stage color, src/Mapper.py:339-341).  When the forward
@@ -141,7 +142,7 @@ typedef struct {
                                     the points of a tile) instead of the FP32-FMA pass that recomputes the forward.  NULL = not kept. */
 } nsb_forward_outputs;
 
-/* 0 when the batch is too large to profit from decoder-parallel CTAs. */
+/* Bytes of split_workspace for n_rays rays of n_samples_total samples (NSB_MAX_SAMPLES: any S up to it); 0 for an empty batch. */
 size_t nsb_split_workspace_bytes(int n_rays, int n_samples_total);
 
 /* Forward: sample -> gather -> decode -> composite  (Renderer.render_batch_ray, src/utils/Renderer.py:63-198) */

@@ -134,18 +134,12 @@ def lib():
         for name, (res, args) in SYMBOLS.items():
             f = getattr(h, name)          # AttributeError if the library does not export a declared symbol
             f.restype, f.argtypes = res, args
-        backend = os.environ.get("NSB_MLP_BACKEND")          # 1 = FP32-FMA decoders, 2 = tcgen05 decoders (default: auto)
+        backend = os.environ.get("NSB_MLP_BACKEND")          # 1 = FP32-FMA decoders (default 0: tile kernels where S >= 8)
         if backend is not None and h.nsb_set_option(b"mlp_backend", int(backend)) != 0:
             raise RuntimeError("bad NSB_MLP_BACKEND=%r" % backend)
-        sr = os.environ.get("NSB_SMALL_RAYS")                # auto back-end: batches up to this many rays use the ray-group kernels
-        if sr is not None and hasattr(h, "nsb_set_option"):
-            h.nsb_set_option(b"small_rays", int(sr))
         wg = os.environ.get("NSB_WGRAD_TC")                  # 0 = decoder weight gradients by the FP32-FMA pass (default: tensor cores)
         if wg is not None:
             h.nsb_set_option(b"wgrad_tc", int(wg))
-        pdl = os.environ.get("NSB_PDL")                      # 0 = plain stream order between the forward and backward launches of an iteration
-        if pdl is not None:
-            h.nsb_set_option(b"pdl", int(pdl))
         f16 = os.environ.get("NSB_FWD_F16")                  # 1 = forward decoders with FP16 hi|lo operands (kind::f16) instead of 3xTF32
         if f16 is not None:
             h.nsb_set_option(b"fwd_f16", int(f16))

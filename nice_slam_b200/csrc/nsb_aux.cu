@@ -81,50 +81,20 @@ __global__ void pack_kernel(const __grid_constant__ PackArgs A) {
 }
 
 // ---- tensor-core operand images (layout: nsb_common.cuh) --------------------------------------------------------------------
-// hi | lo of a [R x 32] canonical tile whose element (row, k) is get(row, k)
-template <typename F>
-__device__ __forceinline__ void emit_tile(float*& dst, int& e, int R, F&& get) {
-  float* hi = dst; float* lo = dst + R * 32;
-  dst += 2 * R * 32;
-  if (!pk_mine(e)) return;
-  for (int idx = threadIdx.x; idx < R * 32; idx += blockDim.x) {
-    const int r = idx >> 5, k = idx & 31;
-    const float v = get(r, k);
-    const float h = __uint_as_float(__float_as_uint(v) & 0xffffe000u);          // the 19 bits the tensor core reads (nsb_tc.cuh)
-    const int o = ((r >> 3) * 8 + (k >> 2)) * 32 + (r & 7) * 4 + (k & 3);
-    hi[o] = h; lo[o] = v - h;
-  }
-}
+// header: biases, output weights and the embedding matrix of one decoder, read by the tile kernels
 template <int LV>
-__device__ void pack_operands_level(float* __restrict__ img /* packed image of this level: raw part already written */, int& e) {
+__device__ void pack_header_level(float* __restrict__ img /* packed image of this level: raw part already written */, int& e) {
   using D = Dec<LV>;
   const float* W = img;
-  constexpr int PH = D::PH;
-  const int o_wh[5] = {0, D::o_W1, D::o_W2, D::o_W3H, D::o_W4};
-  // forward
-  float* dst = img + op_fwd_offset(LV);
+  float* dst = img + op_hdr_offset(LV);
   if (pk_mine(e)) for (int i = threadIdx.x; i < kHdrFloats; i += blockDim.x) {
     float v = 0.0f;
     if (i < 160) v = W[D::o_b + i];
     else if (i < 320) v = D::XYZ ? W[D::o_bc + (i - 160)] : 0.0f;
     else if (i < 324) v = W[D::o_bo + (i - 320)];
-    else if (i >= 336 && i < 464) v = W[D::o_WO + ((i - 336) >> 5) * PH + ((i - 336) & 31)];
+    else if (i >= 336 && i < 464) v = W[D::o_WO + ((i - 336) >> 5) * D::PH + ((i - 336) & 31)];
     else if (i >= 464 && i < 464 + 3 * kEmbPad) v = D::XYZ ? W[D::o_B + (i - 464)] : 0.0f;
     dst[i] = v;
-  }
-  dst += kHdrFloats;
-  if (D::XYZ)
-    for (int h = 0; h < D::CD / 32; h++)
-      emit_tile(dst, e, 160, [&](int r, int k) { return W[D::o_WC + r * D::PC + 32 * h + k]; });          // row r = 32 i + o
-  for (int b = 0; b < op_nblk(LV); b++)
-    emit_tile(dst, e, 64, [&](int r, int k) { return W[(r < 32 ? D::o_W0 : D::o_W3E) + (r & 31) * D::PF + 32 * b + k]; });
-  for (int i = 1; i < 5; i++) emit_tile(dst, e, 32, [&](int r, int k) { return W[o_wh[i] + r * PH + k]; });
-  // backward (transposed operands)
-  dst = img + op_bwd_offset(LV);
-  for (int i = 4; i >= 0; i--) {
-    if (D::XYZ) emit_tile(dst, e, D::CD, [&](int c, int k) { return W[D::o_WC + (i * 32 + k) * D::PC + c]; });
-    if (i >= 1) emit_tile(dst, e, 32, [&](int j, int k) { return W[o_wh[i] + k * PH + j]; });
-    if (i == 3 || i == 0) emit_tile(dst, e, D::FIRSTP, [&](int f, int k) { return W[(i == 0 ? D::o_W0 : D::o_W3E) + k * D::PF + f]; });
   }
 }
 // ---- v2 operand images: units for the tile kernels (layout: nsb_common.cuh op2_*) -------------------------------------------------
@@ -200,10 +170,10 @@ __global__ void pack_operands_kernel(const __grid_constant__ PackArgs A) {
   if (!A.present[lv]) return;
   int e = 0;                                                      // piece counter (pk_mine)
   switch (lv) {
-    case 0: pack_operands_level<0>(A.packed[0], e); pack_units_level<0>(A.packed[0], e); pack_units_h16_level<0>(A.packed[0], e); break;
-    case 1: pack_operands_level<1>(A.packed[1], e); pack_units_level<1>(A.packed[1], e); pack_units_h16_level<1>(A.packed[1], e); break;
-    case 2: pack_operands_level<2>(A.packed[2], e); pack_units_level<2>(A.packed[2], e); pack_units_h16_level<2>(A.packed[2], e); break;
-    default: pack_operands_level<3>(A.packed[3], e); pack_units_level<3>(A.packed[3], e); pack_units_h16_level<3>(A.packed[3], e); break;
+    case 0: pack_header_level<0>(A.packed[0], e); pack_units_level<0>(A.packed[0], e); pack_units_h16_level<0>(A.packed[0], e); break;
+    case 1: pack_header_level<1>(A.packed[1], e); pack_units_level<1>(A.packed[1], e); pack_units_h16_level<1>(A.packed[1], e); break;
+    case 2: pack_header_level<2>(A.packed[2], e); pack_units_level<2>(A.packed[2], e); pack_units_h16_level<2>(A.packed[2], e); break;
+    default: pack_header_level<3>(A.packed[3], e); pack_units_level<3>(A.packed[3], e); pack_units_h16_level<3>(A.packed[3], e); break;
   }
 }
 

@@ -62,33 +62,16 @@ constexpr int kRowsFwd = Dec<2>::ROWS_FWD;     // 160
 constexpr int kRowsBwd = Dec<2>::ROWS_BWD;     // 320
 
 // ---- tensor-core operand images (appended to the packed fp32 image of every decoder by nsb_pack_decoders) -----------------------
-// Every MMA B operand is stored ready to use: the 3xTF32 split (hi | lo) of a [R x 32] K-major no-swizzle canonical tile
-// ([row/8][k/4][row%8][k%4]), in the order the kernels consume them, so one TMA bulk copy per chunk replaces all in-kernel staging.
+// Every MMA B operand is stored ready to use: the 3xTF32 split (hi | lo) of a K-major no-swizzle canonical tile ([row/8][k/4][row%8][k%4]),
+// in the order the kernels consume them, so one TMA bulk copy per unit replaces all in-kernel staging.  Behind the fp32 image:
 //   header (kHdrFloats): b[5][32] | bc[5][32] | bo[4] | pad[12] | Wo[4][32] | B[3][96] | pad
-//   forward : header | FC_h, h < cd/32 : rows 32 i + o = Wc_i[o][32 h + k]            (R = 160: five fc_c layers in one N = 160 MMA)
-//                    | L0_b, b < nblk  : rows o = W0[o][32 b + k], rows 32 + o = W3E[o][32 b + k]   (R = 64: layer 0 and the skip part of layer 3)
-//                    | H_i, i = 1..4   : rows o = W_i[o][hidden k]                               (R = 32)
-//   backward: for i = 4..0:  DC_i : rows c = Wc_i[k][c]  (R = cd, xyz only) | D1_i (i >= 1): rows j = W_i[k][hidden j] (R = 32)
-//                            | DF_i (i = 3, 0): rows f = W_i[k][first-input f] (R = firstp)
+//   | v2 forward units | v2 backward units | v3 forward units (below)
 constexpr int kHdrFloats = 768;
 __host__ __device__ constexpr int op_cd(int lv) { return lv == 2 ? 64 : 32; }
 __host__ __device__ constexpr int op_firstp(int lv) { return lv == 0 ? 32 : kEmbPad; }
 __host__ __device__ constexpr int op_nblk(int lv) { return lv == 0 ? 1 : 3; }
-constexpr int kFcChunk = 2 * 160 * 32, kL0Chunk = 2 * 64 * 32, kHChunk = 2 * 32 * 32;
-__host__ __device__ constexpr int op_fc_floats(int lv) { return lv == 0 ? 0 : (op_cd(lv) / 32) * kFcChunk; }
-__host__ __device__ constexpr int op_fwd_floats(int lv) { return kHdrFloats + op_fc_floats(lv) + op_nblk(lv) * kL0Chunk + 4 * kHChunk; }
-__host__ __device__ constexpr int op_bwd_layer_floats(int lv, int i) {
-  return (lv != 0 ? 2 * op_cd(lv) * 32 : 0) + (i >= 1 ? kHChunk : 0) + ((i == 3 || i == 0) ? 2 * op_firstp(lv) * 32 : 0);
-}
-__host__ __device__ constexpr int op_bwd_layer_offset(int lv, int i) {      // layers are stored 4, 3, 2, 1, 0
-  int off = 0;
-  for (int j = 4; j > i; j--) off += op_bwd_layer_floats(lv, j);
-  return off;
-}
-__host__ __device__ constexpr int op_bwd_floats(int lv) { return op_bwd_layer_offset(lv, -1); }
-__host__ __device__ constexpr int op_fwd_offset(int lv) { return packed_floats(lv); }
-__host__ __device__ constexpr int op_bwd_offset(int lv) { return packed_floats(lv) + op_fwd_floats(lv); }
-// ---- v2 operand images (tile kernels, nsb_tile.cuh): the same matrices cut into UNITS that stream through a 4-slot ring ----------------
+__host__ __device__ constexpr int op_hdr_offset(int lv) { return packed_floats(lv); }
+// ---- v2 operand images (tile kernels, nsb_tile.cuh): the matrices cut into UNITS that stream through a 4-slot ring ----------------
 //   forward : FC_u, u < cd/8   : [160 x 8]  rows 32 i + o = Wc_i[o][8 u + k]                                  (2560 floats hi|lo)
 //             L0_{b,h}, h < 2  : [64 x 16]  rows o = W0[o][32 b + 16 h + k], rows 32 + o = W3E[o][...]          (2048 floats)
 //             H_i, i = 1..4    : [32 x 32]  rows o = W_i[o][hidden k]                                          (2048 floats)
@@ -106,7 +89,7 @@ __host__ __device__ constexpr int op2_bwd_units(int lv) {
   return n;
 }
 __host__ __device__ constexpr int op2_bwd_floats(int lv) { return op2_bwd_units(lv) * 2048; }
-__host__ __device__ constexpr int op2_fwd_offset(int lv) { return packed_floats(lv) + op_fwd_floats(lv) + op_bwd_floats(lv); }
+__host__ __device__ constexpr int op2_fwd_offset(int lv) { return op_hdr_offset(lv) + kHdrFloats; }
 __host__ __device__ constexpr int op2_bwd_offset(int lv) { return op2_fwd_offset(lv) + op2_fwd_floats(lv); }
 // ---- v3 forward image (tile kernels, option fwd_f16): the forward units as FP16 hi | lo pairs (x = hi + lo, hi = fp16(x), lo = fp16(x - hi): the same
 // ~22-bit effective mantissa as the 3xTF32 split at half the bytes; tcgen05 kind::f16 contracts K = 16 per instruction).  16-bit canonical K-major
@@ -117,8 +100,6 @@ __host__ __device__ constexpr int op3_fwd_units(int lv) { return op3_fc_units(lv
 __host__ __device__ constexpr int op3_fwd_floats(int lv) { return op3_fc_units(lv) * 2560 + op_nblk(lv) * 2048 + 4 * 1024; }
 __host__ __device__ constexpr int op3_fwd_offset(int lv) { return op2_bwd_offset(lv) + op2_bwd_floats(lv); }
 __host__ __device__ constexpr int packed_total_floats(int lv) { return op3_fwd_offset(lv) + op3_fwd_floats(lv); }
-constexpr int kBwdStageFloats = op_bwd_layer_floats(2, 3);      // largest backward layer chunk (fine decoder, layer 3): 48 KB
-static_assert(kBwdStageFloats == 12288, "backward stage size");
 
 // canonical flat layout (include/nice_slam_b200.h): kind 0=B 1=W 2=b 3=Wc 4=bc 5=Wo 6=bo 7=total
 __host__ __device__ inline int dec_in(int lv, int i) {
@@ -204,9 +185,7 @@ struct FusedSeeds {
   PeerX px;                      // world > 1: sharded tracking batch -- depth maxima and the median pool are exchanged inside the forward launch
 };
 int render_forward_fused(const nsb_render_inputs* in, const nsb_forward_outputs* out, const FusedSeeds* fs, void* stream);
-// after_forward: the forward launch of the same iteration is the operation right in front of this call on `stream` -> the backward launch may
-// start early (programmatic dependent launch) and run its set-up under the forward's tail
-int render_backward_tail(const nsb_render_inputs* in, const nsb_backward_args* bw, const PeerTail* tail, void* stream, bool after_forward = false);
+int render_backward_tail(const nsb_render_inputs* in, const nsb_backward_args* bw, const PeerTail* tail, void* stream);
 int make_peerx(const struct nsb_peers* p, PeerX* px);
 
 // error plumbing shared by the API translation units

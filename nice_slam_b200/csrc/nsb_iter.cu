@@ -46,14 +46,13 @@ static int forward_part(const nsb_render_inputs* in, const nsb_iteration_buffers
   return render_forward_fused(in2, &fo, fs, stream);
 }
 
-static int backward_part(const nsb_render_inputs* in2, const nsb_iteration_buffers* b, const nsb_backward_args* g, void* stream, const PeerTail* tail = nullptr,
-                         bool after_forward = false) {
+static int backward_part(const nsb_render_inputs* in2, const nsb_iteration_buffers* b, const nsb_backward_args* g, void* stream, const PeerTail* tail = nullptr) {
   nsb_backward_args bw = *g;
   bw.z_vals = b->z_vals; bw.raw = b->raw; bw.g_depth = b->g_depth; bw.g_var = nullptr; bw.g_rgb = b->g_rgb; bw.masks = b->masks; bw.acts = b->acts;
   bw.workspace = reinterpret_cast<char*>(b->workspace) + 16 + a16(nsb_tracking_seeds_workspace(in2->n_rays));
   bw.split_workspace = split_ptr(b, in2->n_rays); bw.split_workspace_bytes = split_room(b, in2->n_rays);
   if (b->event_bwd_begin) cudaEventRecord((cudaEvent_t)b->event_bwd_begin, (cudaStream_t)stream);
-  const int rc = render_backward_tail(in2, &bw, tail, stream, after_forward && !b->event_bwd_begin);
+  const int rc = render_backward_tail(in2, &bw, tail, stream);
   if (b->event_bwd_end) cudaEventRecord((cudaEvent_t)b->event_bwd_end, (cudaStream_t)stream);
   return rc;
 }
@@ -75,7 +74,7 @@ extern "C" int nsb_tracking_iteration(const nsb_render_inputs* in, const nsb_ite
   if ((rc = forward_part(in, buf, &in2, fuse ? &fs : nullptr, stream))) return rc;
   if (!fuse && (rc = nsb_tracking_seeds(buf->depth, buf->var, buf->rgb, in->gt_depth, gt_rgb, in->n_rays, w_color, handle_dynamic, use_color,
                                         nullptr, 0, buf->g_depth, buf->g_rgb, buf->loss, seeds_scratch(buf), nsb_tracking_seeds_workspace(in->n_rays), stream))) return rc;
-  return backward_part(&in2, buf, grads, stream, nullptr, fuse);
+  return backward_part(&in2, buf, grads, stream);
 }
 
 // Ray-sharded tracking iteration in TWO launches per rank: the forward exchanges the depth maxima (every CTA) and the residual pool of the
@@ -99,7 +98,7 @@ extern "C" int nsb_tracking_iteration_peers(const nsb_render_inputs* in, const n
   nsb_render_inputs in2;
   if ((rc = forward_part(in, buf, &in2, &fs, stream, true))) return rc;      // in->depth_max given: no depth-max exchange inside the forward
   PeerTail tail; tail.px = px; tail.loss = buf->loss; tail.out13 = loss_and_d_c2w;
-  return backward_part(&in2, buf, grads, stream, &tail, true);
+  return backward_part(&in2, buf, grads, stream, &tail);
 }
 
 extern "C" int nsb_mapping_iteration(const nsb_render_inputs* in, const nsb_iteration_buffers* buf, const float* gt_depth_loss,
@@ -118,5 +117,5 @@ extern "C" int nsb_mapping_iteration(const nsb_render_inputs* in, const nsb_iter
   }
   if ((rc = forward_part(in, buf, &in2, fuse ? &fs : nullptr, stream))) return rc;
   if (!fuse && (rc = nsb_mapping_seeds(buf->depth, buf->rgb, gtl, gt_rgb, in->n_rays, w_color, use_color, buf->g_depth, buf->g_rgb, buf->loss, stream))) return rc;
-  return backward_part(&in2, buf, grads, stream, nullptr, fuse);
+  return backward_part(&in2, buf, grads, stream);
 }

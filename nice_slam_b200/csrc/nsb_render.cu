@@ -151,13 +151,9 @@ struct KParams {
   int dec[3];
   int dec_pos[3];               // position of dec[i] in the stage's full decoder list (slot of its saved ReLU masks)
   int accumulate_rays;          // backward: add to d_rays_o / d_rays_d instead of overwriting (second launch of a split backward)
-  // decoder-parallel CTAs (tensor-core kernels, small batches): `split` CTAs share one ray group, CTA j evaluates decoder dec[j] only;
-  // their outputs meet in global scratch and the last CTA to arrive (group_done counter) composites / reduces.
-  int split;                    // 1 = one CTA evaluates all decoders of its rays
-  int* group_done;              // [n_groups] arrival counters, zero between launches (the last CTA resets its counter)
-  float4* fwd_parts;            // [n_dec][N*S] decoder outputs of the forward
-  double* ray_parts;            // [n_dec][N][6] per-decoder ray-gradient sums of the backward
   // tile kernels (nsb_tile.cuh): item = (128-point tile, decoder); `split` items per tile
+  int split;                    // 1 = one CTA evaluates all decoders of its tile; n_dec = CTA j of a tile evaluates decoder dec[j] only
+  double* ray_parts;            // backward: [tiles * split][tile_rays][6] per-item ray-gradient sums
   int* ray_cnt;                 // [N] completion counters of the rays, zero between launches (the completing CTA resets them)
   float4* tile_parts;           // forward: [split][N*S] per-item decoder outputs (split == 1: aliases fo.raw)
   int tile_rays;                // backward: rays one tile can touch (stride of ray_parts per item)
@@ -303,7 +299,6 @@ __device__ __forceinline__ void ray_weights(const float* __restrict__ rw, int S,
 // ------------------------------------------------------------------------------------------------
 // forward kernel
 // ------------------------------------------------------------------------------------------------
-// shared by the SIMT and the tensor-core forward kernels
 struct BlockRange { int r0, nr, Pb; };
 __device__ __forceinline__ BlockRange block_range(const KParams& P, int bid) {
   BlockRange b; b.r0 = 0; b.nr = 0;
@@ -473,129 +468,9 @@ __global__ void __launch_bounds__(256, 1) render_fwd_kernel(const __grid_constan
   fused_seeds_tail(P, gridDim.x, smem_raw);
 }
 
-}  // namespace nsb
-#include "nsb_tc.cuh"
-namespace nsb {
-
-// ------------------------------------------------------------------------------------------------
-// forward kernel, tensor-core (tcgen05, 3xTF32) decoders: 512 threads = four per point of a 128-point tile (nsb_tc.cuh)
-__global__ void __launch_bounds__(tc::kThreads, 1) render_fwd_tc_kernel(const __grid_constant__ KParams P) {
-  extern __shared__ __align__(1024) unsigned char smem_raw[];       // tiles need 16-byte alignment only (no-swizzle descriptors)
-  NSB_PH_RESET();
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int row = threadIdx.x & (tc::TM - 1), cg = threadIdx.x >> 7;
-  tc::TcSmem t;
-  tc::tc_carve(smem_raw, t, false);
-  Smem sm;
-  smem_layout(0, P.max_pts, P.max_rays, 0, 0, false, &sm, smem_raw + ((tc::tc_smem_bytes(false) + 127) & ~size_t(127)));
-  const int nsplit = P.split;                                    // decoder-parallel CTAs per ray group (1 = this CTA does all decoders)
-  const int bid = blockIdx.x / nsplit, my = blockIdx.x - bid * nsplit;
-  const int q0 = nsplit > 1 ? my : 0, q1 = nsplit > 1 ? my + 1 : P.n_dec;
-  const BlockRange b = block_range(P, bid);
-  const int Pb = b.Pb;
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(t.tmem)), "r"(tc::kTmemCols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc::Pipe pp; pp.par = 0; pp.hb = 0; pp.prefetched = true;
-  if (threadIdx.x == 0) {
-    for (int i = 0; i < tc::kNumBarsFwd; i++) mbar_init(t.bars + i, 1);
-    mbar_fence_init();
-    tc::issue_fwd_loads(P, t, P.dec[q0], 0);                     // the first decoder's weights arrive under the sampling prologue
-  }
-  fwd_sample_sort(P, sm, b);                                     // contains __syncthreads(): TMEM address + barriers are visible after it
-  tc::tc_fence_before();
-  __syncthreads();
-  tc::tc_fence_after();
-  const uint32_t tmem = *t.tmem;
-  NSB_PH(13);                                                    // sampling / sorting prologue (mark 0 of the first decoder closes it)
-
-  const int ntiles = (Pb + tc::TM - 1) / tc::TM;
-  for (int tile = 0; tile < ntiles; tile++) {
-    const int lp = tile * tc::TM + row;
-    const int lpc = lp < Pb ? lp : Pb - 1;
-    PointGeom G;
-    if (P.points != nullptr) {
-      const long long gp = (long long)bid * P.rays_per_block + lpc;
-      const double pin[3] = {P.points[3 * gp], P.points[3 * gp + 1], P.points[3 * gp + 2]};
-      make_point_from_p(P.in.bound, P.in.coarse_bound, pin, G);
-    } else {
-      const int ray = lpc / P.S;
-      const float* rr = sm.rays + 8 * ray;
-      const float o[3] = {rr[0], rr[1], rr[2]}, dd[3] = {rr[3], rr[4], rr[5]};
-      make_point(P.in.bound, P.in.coarse_bound, o, dd, sm.zs[lpc], G);
-    }
-    const long long gp0 = ((long long)bid * P.rays_per_block) * P.S;             // global index of this CTA's first point
-    float occ = 0.0f, c0 = 0.0f, c1 = 0.0f, c2 = 0.0f;
-    for (int qd = q0; qd < q1; qd++) {
-      const int lv = P.dec[qd];
-      const DecRT d = make_dec(lv);
-      float out[4];
-      uint32_t* gm = (P.fo.masks != nullptr && lp < Pb) ? P.fo.masks + ((gp0 + lp) * 15 + qd * 5) : nullptr;
-      const int next_lv = qd + 1 < q1 ? P.dec[qd + 1] : (tile + 1 < ntiles ? P.dec[q0] : -1);
-      tc::tile_forward(P, t, d, lv, G, tmem, pp, out, gm, next_lv);
-      if (lv == 3) { c0 = out[0]; c1 = out[1]; c2 = out[2]; } else occ += out[0];
-      if (nsplit > 1 && cg == 0 && lp < Pb)                                     // this decoder's outputs -> global scratch
-        P.fwd_parts[(long long)qd * P.in.n_rays * P.S + gp0 + lp] = make_float4(out[0], out[1], out[2], out[3]);
-      if (qd == 0 && cg == 0 && lp < Pb && P.fo.corner_idx != nullptr) {
-        const nsb_grid& g = P.in.grid[lv];
-        const Tri tr = make_tri(lv == 0 ? G.xnc : G.xn, g.W, g.H, g.D);
-        const long long gp = gp0 + lp;
-        P.fo.corner_idx[3 * gp] = tr.i0[0]; P.fo.corner_idx[3 * gp + 1] = tr.i0[1]; P.fo.corner_idx[3 * gp + 2] = tr.i0[2];
-      }
-    }
-    if (cg == 0 && lp < Pb) {
-      *reinterpret_cast<float4*>(sm.raw + 4 * lp) = make_float4(c0, c1, c2, occ);
-      sm.inb[lp] = (unsigned char)G.inb;
-    }
-  }
-  tc::tc_fence_before();
-  __syncthreads();
-  if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(tc::kTmemCols) : "memory");
-  if (nsplit > 1) {
-    // decoder-parallel CTAs: the last CTA of the ray group to arrive gathers every decoder's outputs and composites
-    __shared__ int s_last;
-    __threadfence();
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      const int old = atomicAdd(P.group_done + bid, 1);
-      s_last = old == nsplit - 1;
-      if (s_last) P.group_done[bid] = 0;                           // everybody has arrived: leave the counter clean for the next launch
-    }
-    __syncthreads();
-    if (!s_last) return;
-    __threadfence();
-    const long long gp0 = ((long long)bid * P.rays_per_block) * P.S, NS = (long long)P.in.n_rays * P.S;
-    for (int lp = threadIdx.x; lp < Pb; lp += blockDim.x) {
-      float c0 = 0.0f, c1 = 0.0f, c2 = 0.0f, occ = 0.0f;
-      for (int q = 0; q < P.n_dec; q++) {                          // same order as the single-CTA path: occ = fine + middle
-        const float4 v = __ldcg(P.fwd_parts + q * NS + gp0 + lp);
-        if (P.dec[q] == 3) { c0 = v.x; c1 = v.y; c2 = v.z; } else occ += v.x;
-      }
-      *reinterpret_cast<float4*>(sm.raw + 4 * lp) = make_float4(c0, c1, c2, occ);
-    }
-    __syncthreads();
-  }
-  NSB_PH(14);
-  fwd_composite_store(P, sm, b, warp, tc::kThreads / 32, lane);
-  NSB_PH(15);
-  fused_seeds_tail(P, gridDim.x / nsplit, smem_raw);             // (split launches: one participant per ray group, the compositing CTA)
-}
-
 // ------------------------------------------------------------------------------------------------
 // backward kernel
 // ------------------------------------------------------------------------------------------------
-// sharded tracking batch: SUM over ranks of [loss | d c2w] by the (last) CTA that just reduced the pose gradient -- identical bits on every rank
-__device__ __forceinline__ void pose_tail_peers(const KParams& P) {
-  if (P.tail.px.world <= 1) return;
-  __shared__ double tot[13];
-  __shared__ uint32_t s_seq2;
-  __syncthreads();
-  if (threadIdx.x == 0) tot[0] = P.tail.loss != nullptr ? P.tail.loss[0] : 0.0;
-  if (threadIdx.x < 12) tot[1 + threadIdx.x] = P.bw.d_c2w[threadIdx.x];
-  __syncthreads();
-  peer_sum13(P.tail.px, tot, 13, P.tail.out13, &s_seq2);
-}
 __device__ __forceinline__ void chunk_backward(const KParams& P, const Smem& sm, float* act, int chunk, int Pb,
                                                const LaneId& L, uint32_t parity, const float* gC /*[R][3] smem*/,
                                                const int lv, const DecRT& d) {
@@ -640,7 +515,7 @@ __device__ __forceinline__ void chunk_backward(const KParams& P, const Smem& sm,
   __syncwarp();
 }
 
-// shared by the SIMT and tensor-core backward kernels: load the forward state, in-bound flags, and the per-ray scans
+// load the forward state, in-bound flags, and the per-ray scans
 __device__ __forceinline__ void bwd_prologue(const KParams& P, const Smem& sm, int r0, int nr, int Pb, int warp, int warps, int lane, float* gC) {
   const long long g0 = (long long)r0 * P.S;
   block_setup_rays(P, sm, r0, nr, 0.0f);                         // only o, d are used below (z comes from forward)
@@ -808,128 +683,8 @@ __global__ void __launch_bounds__(256, 1) render_bwd_kernel(const __grid_constan
   bwd_ray_reduce(P, sm, r0, nr);
 }
 
-// ------------------------------------------------------------------------------------------------
-// backward kernel, tensor-core decoders (input gradients: rays + grid voxels).  Decoder-weight gradients stay on the
-// SIMT kernel for now (host dispatch).
-__global__ void __launch_bounds__(tc::kThreads, 1) render_bwd_tc_kernel(const __grid_constant__ KParams P) {
-  extern __shared__ __align__(1024) unsigned char smem_raw[];
-  NSB_PH_RESET();
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int row = threadIdx.x & (tc::TM - 1);
-  tc::TcSmem t;
-  tc::tc_carve(smem_raw, t, true);
-  Smem sm;
-  smem_layout(0, P.max_pts, P.max_rays, 0, 0, true, &sm, smem_raw + ((tc::tc_smem_bytes(true) + 127) & ~size_t(127)));
-  __shared__ float gC[kMaxRaysPerBlock * 3];
-  const int nsplit = P.split;                                    // decoder-parallel CTAs per ray group
-  const int bid = blockIdx.x / nsplit, my = blockIdx.x - bid * nsplit;
-  const int q0 = nsplit > 1 ? my : 0, q1 = nsplit > 1 ? my + 1 : P.n_dec;
-  const int r0 = bid * P.rays_per_block;
-  const int nr = P.in.n_rays - r0 < P.rays_per_block ? P.in.n_rays - r0 : P.rays_per_block;
-  const int Pb = nr * P.S;
-  if (warp == 0) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(t.tmem)), "r"(tc::kTmemCols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc::Pipe pp; pp.par = 0; pp.hb = 0; pp.prefetched = true;
-  if (threadIdx.x == 0) {
-    for (int i = 0; i < tc::kNumBarsBwd; i++) mbar_init(t.bars + i, 1);
-    mbar_fence_init();
-    tc::issue_bwd_loads(P, t, P.dec[q0], 0);                     // the first decoder's operands arrive under the compositing prologue
-  }
-  bwd_prologue(P, sm, r0, nr, Pb, warp, tc::kThreads / 32, lane, gC);
-  tc::tc_fence_before();
-  __syncthreads();
-  tc::tc_fence_after();
-  const uint32_t tmem = *t.tmem;
-
-  const int ntiles = (Pb + tc::TM - 1) / tc::TM;
-  for (int tile = 0; tile < ntiles; tile++) {
-    const int lp = tile * tc::TM + row;
-    const int lpc = lp < Pb ? lp : Pb - 1;
-    const int ray = lpc / P.S;
-    PointGeom G;
-    {
-      const float* rr = sm.rays + 8 * ray;
-      const float o[3] = {rr[0], rr[1], rr[2]}, dd[3] = {rr[3], rr[4], rr[5]};
-      make_point(P.in.bound, P.in.coarse_bound, o, dd, sm.zs[lpc], G);
-    }
-    for (int qd = q0; qd < q1; qd++) {
-      const int lv = P.dec[qd];
-      const DecRT d = make_dec(lv);
-      const uint32_t* gm = P.bw.masks + ((((long long)bid * P.rays_per_block) * P.S + lpc) * 15 + P.dec_pos[qd] * 5);   // saved by the forward kernel
-      float g_out[4] = {0.f, 0.f, 0.f, 0.f};
-      if (lp < Pb) {
-        if (lv == 3) { const float w = sm.wgt[lp]; g_out[0] = w * gC[3 * ray]; g_out[1] = w * gC[3 * ray + 1]; g_out[2] = w * gC[3 * ray + 2]; }
-        else g_out[0] = sm.gocc[lp];
-      }
-      const int next_lv = qd + 1 < q1 ? P.dec[qd + 1] : (tile + 1 < ntiles ? P.dec[q0] : -1);
-      tc::tile_backward(P, t, d, lv, G, tmem, pp, g_out, gm, next_lv);
-      __syncthreads();                                           // dL/dc rows + the embedding partials are visible
-      NSB_PH(28);
-      const double* bb = lv == 0 ? P.in.coarse_bound : P.in.bound;
-      const double sc[3] = {2.0 / (bb[1] - bb[0]), 2.0 / (bb[3] - bb[2]), 2.0 / (bb[5] - bb[4])};      // d(normalised)/dp, common.py:280-282
-      const float* xn = lv == 0 ? G.xnc : G.xn;
-      // one writer per point: dL/dp = embedding chain (partials of tile_backward) + trilinear-coordinate chain of this grid
-      tc::scatter_rows(P.in.grid[lv], P.bw.d_grid[lv], P.bw.slot_map[lv], t.x, d.cd, xn, warp, lane, [&](int prow, const float gx[3]) {
-        const int l2 = tile * tc::TM + prow;
-        if (l2 < Pb) {
-          float dpe[3];
-          tc::dpe_sum(t, prow, dpe);
-#pragma unroll
-          for (int a = 0; a < 3; a++) sm.dp[3 * l2 + a] += (double)dpe[a] + (double)gx[a] * sc[a];
-        }
-      });
-      NSB_PH(29);
-    }
-  }
-  tc::tc_fence_before();
-  __syncthreads();
-  if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(tc::kTmemCols) : "memory");
-  if (nsplit > 1) {
-    // decoder-parallel CTAs: per-decoder ray sums -> global scratch; the last CTA of the group adds them in decoder order
-    __shared__ int s_last;
-    for (int i = threadIdx.x; i < nr * 3; i += blockDim.x) {
-      const int r = i / 3, a = i - 3 * r;
-      double so = 0.0, sd = 0.0;
-      for (int s = 0; s < P.S; s++) { const double v = sm.dp[3 * (r * P.S + s) + a]; so += v; sd += v * sm.zs[r * P.S + s]; }
-      double* part = P.ray_parts + ((long long)my * P.in.n_rays + r0 + r) * 6;
-      part[a] = so; part[3 + a] = sd;
-    }
-    __threadfence();
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      const int old = atomicAdd(P.group_done + bid, 1);
-      s_last = old == nsplit - 1;
-      if (s_last) P.group_done[bid] = 0;
-    }
-    __syncthreads();
-    if (!s_last) return;
-    __threadfence();
-    for (int i = threadIdx.x; i < nr * 3; i += blockDim.x) {
-      const int r = i / 3, a = i - 3 * r;
-      double so = 0.0, sd = 0.0;
-      for (int q = 0; q < nsplit; q++) {
-        const double* part = P.ray_parts + ((long long)q * P.in.n_rays + r0 + r) * 6;
-        so += __ldcg(part + a); sd += __ldcg(part + 3 + a);
-      }
-      if (P.accumulate_rays) {
-        if (P.bw.d_rays_o != nullptr) so += (double)P.bw.d_rays_o[3 * (r0 + r) + a];
-        if (P.bw.d_rays_d != nullptr) sd += (double)P.bw.d_rays_d[3 * (r0 + r) + a];
-      }
-      if (P.bw.d_rays_o != nullptr) P.bw.d_rays_o[3 * (r0 + r) + a] = (float)so;
-      if (P.bw.d_rays_d != nullptr) P.bw.d_rays_d[3 * (r0 + r) + a] = (float)sd;
-    }
-    if (fused_pose_grad(P, gridDim.x / nsplit, reinterpret_cast<double*>(smem_raw))) pose_tail_peers(P);     // one arrival per ray group (the tiles are dead)
-    return;
-  }
-  bwd_ray_reduce(P, sm, r0, nr);
-  __syncthreads();
-  if (fused_pose_grad(P, gridDim.x, reinterpret_cast<double*>(smem_raw))) pose_tail_peers(P);
-  NSB_PH(30);
-}
-
 }  // namespace nsb
+#include "nsb_tc.cuh"
 #include "nsb_tile.cuh"
 namespace nsb {
 
@@ -976,7 +731,7 @@ static void fill_common(KParams& K, const nsb_render_inputs* in) {
   K.n_dec = stage_decoders(in->stage, K.dec);
   for (int i = 0; i < 3; i++) K.dec_pos[i] = i;
   K.accumulate_rays = 0;
-  K.split = 1; K.group_done = nullptr; K.fwd_parts = nullptr; K.ray_parts = nullptr; K.ray_cnt = nullptr; K.tile_parts = nullptr; K.tile_rays = 0;
+  K.split = 1; K.ray_parts = nullptr; K.ray_cnt = nullptr; K.tile_parts = nullptr; K.tile_rays = 0;
   memset(&K.fs, 0, sizeof(K.fs)); memset(&K.tail, 0, sizeof(K.tail));
   int wb = 0;
   for (int i = 0; i < K.n_dec; i++) { const int b = packed_floats(K.dec[i]) * 4; wb = b > wb ? b : wb; }
@@ -999,11 +754,9 @@ static int sm_count() {
 // choose rays per CTA and warps per CTA: fill all SMs once before growing CTAs (latency-bound small batches),
 // cap CTA size by the shared-memory budget (227 KB per CTA, 1 KB kept for static shared memory)
 constexpr size_t kSmemCap = 226u * 1024u;
-constexpr int kMaxPtsTc = 256;            // points per CTA of the tensor-core kernels (2 tiles)
-static void choose_config(int n_items, int S, int rows, bool bwd, int wbytes, int max_warps, KParams* K, int* warps, size_t* smem,
-                          int max_pts_cap = kMaxPtsPerBlock) {
+static void choose_config(int n_items, int S, int rows, bool bwd, int wbytes, int max_warps, KParams* K, int* warps, size_t* smem) {
   const int sms = sm_count();
-  int r_cap = max_pts_cap / S; if (r_cap < 1) r_cap = 1; if (r_cap > kMaxRaysPerBlock) r_cap = kMaxRaysPerBlock;
+  int r_cap = kMaxPtsPerBlock / S; if (r_cap < 1) r_cap = 1; if (r_cap > kMaxRaysPerBlock) r_cap = kMaxRaysPerBlock;
   int r = (n_items + sms - 1) / sms; if (r < 1) r = 1; if (r > r_cap) r = r_cap;
   const int max_pts = ((r * S + kChunk - 1) / kChunk) * kChunk;
   const int chunks = max_pts / kChunk;
@@ -1017,22 +770,9 @@ static void choose_config(int n_items, int S, int rows, bool bwd, int wbytes, in
 }
 
 static int g_split_model = 1;      // tile kernels: per-decoder items only while they beat all-decoder items by wave efficiency (0: split whenever N*S <= kSplitMaxPts)
-static int g_pdl = 0;              // iteration entry points: the backward launch as a programmatic dependent of the forward launch
 static int g_fwd_f16 = 0;          // tile-kernel forward with FP16 hi|lo operands (kind::f16, K = 16 per MMA) instead of 3xTF32; see nsb_tile.cuh mma_unit_h
 static int g_wgrad_tc = 1;         // decoder weight gradients on the tensor cores when the forward kept the layer outputs (0: FP32-FMA pass)
-static int g_mlp_backend = 0;      // 0 = auto (tensor-core forward), 1 = SIMT, 2 = tcgen05
-static size_t tc_total_smem(int max_pts, int max_rays, bool bwd = false) {
-  return ((tc::tc_smem_bytes(bwd) + 127) & ~size_t(127)) + smem_layout(0, max_pts, max_rays, 0, 0, bwd, nullptr, nullptr);
-}
-
-// ---- decoder-parallel CTAs: workspace layout and launch policy ------------------------------------------------------------------
-constexpr int kSplitMaxRays = 256;
-static size_t split_counters_bytes(int n_rays) { return align16((size_t)n_rays * sizeof(int)); }
-static size_t old_split_workspace_bytes(int n_rays, int S) {
-  if (n_rays < 1 || n_rays > kSplitMaxRays || S < 1) return 0;
-  const size_t fwd = (size_t)3 * n_rays * S * sizeof(float4), bwd = (size_t)3 * n_rays * 6 * sizeof(double);
-  return split_counters_bytes(n_rays) + (fwd > bwd ? fwd : bwd);
-}
+static int g_mlp_backend = 0;      // 0 = auto (tile kernels where S >= 8, otherwise FP32-FMA), 1 = FP32-FMA
 // ---- tile kernels: workspace = [16 B | ray completion counters (N ints) | per-item scratch] -----------------------------------------
 // per-item scratch: forward = decoder outputs [split][N*S] float4 (only when items are split per decoder; otherwise they live in fo.raw),
 // backward = ray-gradient parts [tiles * split][kMaxTileRays][6] f64.  Items are split per decoder for batches of up to kSplitMaxPts points
@@ -1084,55 +824,17 @@ extern "C" size_t nsb_split_workspace_bytes(int n_rays, int S) {
   };
   size_t m = need(S);
   if (S >= NSB_MAX_SAMPLES) for (int s = tl::kMinSamples; s < NSB_MAX_SAMPLES; s++) { const size_t v = need(s); if (v > m) m = v; }   // "any S" sizing (nsb_iteration_workspace_bytes)
-  m += 16 + align16((size_t)n_rays * sizeof(int));
-  const size_t old = old_split_workspace_bytes(n_rays, S);
-  return m > old ? m : old;
+  return m + 16 + align16((size_t)n_rays * sizeof(int));
 }
-// Decide whether `nd` CTAs per ray group beat one.  Cost model = tiles a CTA walks through x decoders it evaluates x waves.
-// On success K->rays_per_block / max_pts / max_rays / split and the scratch pointers are set.
-static bool plan_split(KParams* K, int nd, void* ws, size_t ws_bytes) {
-  const int N = K->in.n_rays, S = K->S;
-  if (nd < 2 || K->points != nullptr || !ws || N > kSplitMaxRays || ws_bytes < old_split_workspace_bytes(N, S) || (reinterpret_cast<uintptr_t>(ws) & 15)) return false;
-  const int sms = sm_count();
-  int r_cap = kMaxPtsTc / S; if (r_cap < 1) return false; if (r_cap > kMaxRaysPerBlock) r_cap = kMaxRaysPerBlock;
-  int r1 = 0;
-  for (int r = 1; r <= r_cap; r++) if (((N + r - 1) / r) * nd <= sms) { r1 = r; break; }
-  if (!r1) return false;
-  auto tiles = [&](int r) { return (r * S + tc::TM - 1) / tc::TM; };
-  const int groups0 = (N + K->rays_per_block - 1) / K->rays_per_block;
-  const int cost0 = ((groups0 + sms - 1) / sms) * tiles(K->rays_per_block) * nd, cost1 = tiles(r1);
-  if (cost1 >= cost0) return false;
-  K->rays_per_block = r1; K->max_rays = r1; K->max_pts = ((r1 * S + kChunk - 1) / kChunk) * kChunk;
-  K->split = nd;
-  K->group_done = static_cast<int*>(ws);
-  char* rest = static_cast<char*>(ws) + split_counters_bytes(N);
-  K->fwd_parts = reinterpret_cast<float4*>(rest);
-  K->ray_parts = reinterpret_cast<double*>(rest);
-  return true;
-}
-
 static size_t tile_smem_bytes(bool bwd) { return tl::common_bytes(bwd) + (bwd ? sizeof(tl::BwdExtra) : 0); }
 static size_t tile_wg_smem_bytes() { return tl::kWgBytes + ((tile_smem_bytes(true) + 1023) & ~size_t(1023)) + 1024; }
-// Which tensor-core kernel family serves a launch.  mlp_backend 3: always the tile kernels; 2: always the round-1 ray-group kernels; 0 (auto): the
-// tile kernels, except that batches of up to g_small_rays rays go to the ray-group kernels (option "small_rays"; default 0 = never: since the
-// channels-last gather became straight-line code the tile kernels are level with them at 200 rays -- 0.1105 ms per tracking iteration either way,
-// r02j / r02l -- and ahead everywhere else).  Forward and backward of an iteration see the same (S, n_rays) and so pick the same family (the saved
-// ReLU bits are laid out per family).
-static int g_small_rays = 0;
-static bool use_tile_kernels(int S, int n_rays, bool sharded) {
-  if (!(g_mlp_backend == 0 || g_mlp_backend == 3) || S < tl::kMinSamples || S > NSB_MAX_SAMPLES) return false;
-  if (g_mlp_backend == 0 && n_rays <= g_small_rays && S <= kMaxPtsTc) return false;
-  return true;
-}
-static bool use_group_kernels(int S, int n_rays, bool sharded) {
-  return S <= kMaxPtsTc && (g_mlp_backend == 2 || (g_mlp_backend == 0 && !use_tile_kernels(S, n_rays, sharded)));
-}
+// Tensor-core tile kernels or FP32-FMA kernels.  A tile may touch at most kMaxTileRays rays, which bounds S from below; smaller S runs on the
+// FP32-FMA kernels.  Forward and backward of an iteration see the same S and so pick the same family (the saved ReLU bits are laid out per family).
+static bool use_tile_kernels(int S) { return g_mlp_backend == 0 && S >= tl::kMinSamples && S <= NSB_MAX_SAMPLES; }
 static bool g_attr_set[kMaxDevices] = {false};
 static int set_attrs() {
   const int dev = current_device();
   if (g_attr_set[dev]) return NSB_OK;
-  if (check_cuda(cudaFuncSetAttribute(render_fwd_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemCap), "fwd tc smem attr")) return NSB_ERR_CUDA;
-  if (check_cuda(cudaFuncSetAttribute(render_bwd_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemCap), "bwd tc smem attr")) return NSB_ERR_CUDA;
   if (check_cuda(cudaFuncSetAttribute(render_fwd_tile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tile_smem_bytes(false)), "fwd tile smem attr")) return NSB_ERR_CUDA;
   if (check_cuda(cudaFuncSetAttribute(render_fwd_tile_h16_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)tile_smem_bytes(false)), "fwd tile (f16) smem attr")) return NSB_ERR_CUDA;
   if (check_cuda(cudaFuncSetAttribute(render_fwd_tile_h16_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, (int)cudaSharedmemCarveoutMaxShared), "fwd tile (f16) carveout")) return NSB_ERR_CUDA;
@@ -1154,10 +856,8 @@ using namespace nsb;
 extern "C" int nsb_set_option(const char* key, int value) {
   if (key && !strcmp(key, "wgrad_tc")) { g_wgrad_tc = value != 0; return NSB_OK; }
   if (key && !strcmp(key, "fwd_f16")) { g_fwd_f16 = value != 0; return NSB_OK; }
-  if (key && !strcmp(key, "pdl")) { g_pdl = value != 0; return NSB_OK; }
   if (key && !strcmp(key, "split_model")) { g_split_model = value != 0; return NSB_OK; }
-  if (key && !strcmp(key, "small_rays")) { if (value < 0) { set_error("small_rays must be >= 0"); return NSB_ERR_ARG; } g_small_rays = value; return NSB_OK; }
-  if (key && !strcmp(key, "mlp_backend")) { if (value < 0 || value > 3) { set_error("mlp_backend must be 0 (auto = tile kernels), 1 (FP32-FMA), 2 (tcgen05, round-1 ray-group kernels) or 3 (tcgen05 tile kernels)"); return NSB_ERR_ARG; } g_mlp_backend = value; return NSB_OK; }
+  if (key && !strcmp(key, "mlp_backend")) { if (value < 0 || value > 1) { set_error("mlp_backend must be 0 (auto = tile kernels) or 1 (FP32-FMA)"); return NSB_ERR_ARG; } g_mlp_backend = value; return NSB_OK; }
   set_error("unknown option %s", key ? key : "(null)"); return NSB_ERR_ARG;
 }
 
@@ -1170,14 +870,13 @@ int nsb::render_forward_fused(const nsb_render_inputs* in, const nsb_forward_out
   if (in->n_rays == 0) return NSB_OK;
   KParams K; fill_common(K, in); K.fo = *out; memset(&K.bw, 0, sizeof(K.bw));
   if (fs != nullptr) K.fs = *fs;
-  const bool sharded = fs != nullptr && fs->px.world > 1;
-  const bool tile = use_tile_kernels(K.S, in->n_rays, sharded), group = use_group_kernels(K.S, in->n_rays, sharded);
-  if (!tile && !group) K.fo.masks = nullptr;                      // only the tensor-core forwards produce masks
+  const bool tile = use_tile_kernels(K.S);
+  if (!tile) K.fo.masks = nullptr;                                // only the tensor-core forward produces masks
   if (K.S > NSB_MAX_SAMPLES) { set_error("n_samples+n_surface = %d exceeds %d", K.S, NSB_MAX_SAMPLES); return NSB_ERR_UNSUPPORTED; }
   if (K.has_gt && in->n_surface > 0 && !in->t_surface) { set_error("t_surface NULL"); return NSB_ERR_ARG; }
   if ((rc = set_attrs())) return rc;
-  if (K.fs.px.world > 1 && !((tile || group) && in->gt_depth != nullptr)) {
-    set_error("in-kernel exchanges of a sharded forward need a tensor-core back-end and <= %d rays per rank", NSB_INLINE_MAX_RAYS); return NSB_ERR_UNSUPPORTED; }
+  if (K.fs.px.world > 1 && !(tile && in->gt_depth != nullptr)) {
+    set_error("in-kernel exchanges of a sharded forward need the tile kernels (mlp_backend 0, n_samples+n_surface >= %d) and gt_depth", tl::kMinSamples); return NSB_ERR_UNSUPPORTED; }
   if (tile) {                                             // tile kernels: item = (128-point tile, decoder), two CTAs per SM
     if (!out->z_vals || !out->raw) { set_error("the tensor-core forward needs z_vals and raw outputs"); return NSB_ERR_ARG; }
     TileWs w;
@@ -1194,15 +893,6 @@ int nsb::render_forward_fused(const nsb_render_inputs* in, const nsb_forward_out
   choose_config(in->n_rays, K.S, kRowsFwd, false, K.wbytes, 8, &K, &warps, &smem);
   if (smem > kSmemCap) { set_error("shared-memory budget exceeded (%zu bytes)", smem); return NSB_ERR_UNSUPPORTED; }
   const int grid = (in->n_rays + K.rays_per_block - 1) / K.rays_per_block;
-  if (group) {                                            // tensor-core decoders, 512 threads, <= 2 tiles of 128 points per CTA
-    choose_config(in->n_rays, K.S, kRowsFwd, false, K.wbytes, 8, &K, &warps, &smem, kMaxPtsTc);
-    plan_split(&K, K.n_dec, out->split_workspace, out->split_workspace_bytes);
-    const int grid_tc = ((in->n_rays + K.rays_per_block - 1) / K.rays_per_block) * K.split;
-    const size_t smem_tc = tc_total_smem(K.max_pts, K.max_rays);
-    if (smem_tc > kSmemCap) { set_error("shared-memory budget exceeded (%zu bytes)", smem_tc); return NSB_ERR_UNSUPPORTED; }
-    render_fwd_tc_kernel<<<grid_tc, tc::kThreads, smem_tc, (cudaStream_t)stream>>>(K);
-    return check_cuda(cudaGetLastError(), "render_fwd_tc_kernel launch");
-  }
   render_fwd_kernel<<<grid, warps * 32, smem, (cudaStream_t)stream>>>(K);
   return check_cuda(cudaGetLastError(), "render_fwd_kernel launch");
 }
@@ -1224,15 +914,11 @@ extern "C" int nsb_eval_points(const nsb_render_inputs* in, const double* points
   const size_t smem = smem_layout(K.wbytes, ppb, 1, warps, kRowsFwd, false, nullptr, nullptr);
   K.rays_per_block = ppb; K.max_pts = ppb; K.max_rays = 1;
   const int grid = (n_points + ppb - 1) / ppb;
-  if (g_mlp_backend == 0 || g_mlp_backend == 3) {
+  if (g_mlp_backend == 0) {
     K.split = 1;
     if (g_fwd_f16) render_fwd_tile_h16_kernel<<<(unsigned)tile_count(n_points), tl::kThreads, tile_smem_bytes(false), (cudaStream_t)stream>>>(K);
     else render_fwd_tile_kernel<<<(unsigned)tile_count(n_points), tl::kThreads, tile_smem_bytes(false), (cudaStream_t)stream>>>(K);
     return check_cuda(cudaGetLastError(), "render_fwd_tile_kernel(points) launch");
-  }
-  if (g_mlp_backend == 2) {
-    render_fwd_tc_kernel<<<grid, tc::kThreads, tc_total_smem(K.max_pts, K.max_rays), (cudaStream_t)stream>>>(K);
-    return check_cuda(cudaGetLastError(), "render_fwd_tc_kernel(points) launch");
   }
   render_fwd_kernel<<<grid, warps * 32, smem, (cudaStream_t)stream>>>(K);
   return check_cuda(cudaGetLastError(), "render_fwd_kernel(points) launch");
@@ -1245,9 +931,9 @@ extern "C" size_t nsb_backward_workspace_bytes(void) {
 }
 
 extern "C" int nsb_render_backward(const nsb_render_inputs* in, const nsb_backward_args* bw, void* stream) {
-  return nsb::render_backward_tail(in, bw, nullptr, stream, false);
+  return nsb::render_backward_tail(in, bw, nullptr, stream);
 }
-int nsb::render_backward_tail(const nsb_render_inputs* in, const nsb_backward_args* bw, const nsb::PeerTail* tail, void* stream, bool after_forward) {
+int nsb::render_backward_tail(const nsb_render_inputs* in, const nsb_backward_args* bw, const nsb::PeerTail* tail, void* stream) {
   int rc = validate_inputs(in, true); if (rc) return rc;
   if (!bw || !bw->z_vals || !bw->raw) { set_error("backward needs z_vals and raw from the forward pass"); return NSB_ERR_ARG; }
   if (in->n_rays == 0) return NSB_OK;
@@ -1287,8 +973,7 @@ int nsb::render_backward_tail(const nsb_render_inputs* in, const nsb_backward_ar
   choose_config(in->n_rays, K.S, kRowsBwd, true, K.wbytes, 8, &K, &warps, &smem);
   if (smem > kSmemCap) { set_error("shared-memory budget exceeded (%zu bytes)", smem); return NSB_ERR_UNSUPPORTED; }
   const bool sharded = tail != nullptr && tail->px.world > 1;
-  const bool tile = use_tile_kernels(K.S, in->n_rays, sharded), group = use_group_kernels(K.S, in->n_rays, sharded);
-  if (bw->masks != nullptr && (group || tile)) {                  // (no saved ReLU masks -> FP32 kernel, which recomputes the forward)
+  if (bw->masks != nullptr && use_tile_kernels(K.S)) {            // (no saved ReLU masks -> FP32 kernel, which recomputes the forward)
     // Tensor-core kernel for the decoders that only need input gradients (rays, voxels).  Decoders whose WEIGHT gradients are
     // requested (the colour decoder in the mapper's colour stage, Mapper.py:339-341) go through the FP32-FMA kernel in a second
     // launch that adds its share of the ray gradients.
@@ -1301,47 +986,20 @@ int nsb::render_backward_tail(const nsb_render_inputs* in, const nsb_backward_ar
     }
     // Weight gradients on the tensor cores: the colour decoder, when the forward kept its layer outputs (acts) -- a second tile launch with one item
     // per tile (one CTA per SM) after the input-gradient launch of the other decoders; it adds its share of the ray gradients.
-    const bool wg_tc = n_w == 1 && wdec[0] == 3 && bw->acts != nullptr && tile && g_wgrad_tc && !sharded;
+    const bool wg_tc = n_w == 1 && wdec[0] == 3 && bw->acts != nullptr && g_wgrad_tc && !sharded;
     if (T.n_dec > 0) {
       if (n_w == 0 && want_pose) T.bw.pose_dirs = bw->pose_dirs;   // the tensor-core launch is the last writer of the ray gradients
-      if (tile) {
-        TileWs w;
-        if (!tile_ws_plan(bw->split_workspace, bw->split_workspace_bytes, in->n_rays, T.S, T.n_dec, true, &w)) {
-          set_error("split_workspace missing or smaller than nsb_split_workspace_bytes(%d, %d)", in->n_rays, T.S); return NSB_ERR_ARG; }
-        T.split = w.split; T.ray_cnt = w.ray_cnt; T.ray_parts = static_cast<double*>(w.scratch); T.tile_rays = tile_rays(T.S);
-        if (tail != nullptr && tail->px.world > 1) {
-          if (n_w != 0 || T.bw.pose_dirs == nullptr) { set_error("sharded backward tail needs pose_dirs and no decoder weight gradients"); return NSB_ERR_ARG; }
-          T.tail = *tail;
-        }
-        const long long grid_t = tile_count((long long)in->n_rays * T.S) * T.split;
-        if (after_forward && !any_w && g_pdl) {
-          // Programmatic dependent launch: the forward kernel signals `launch_dependents` when it starts, so this grid's CTAs become resident as
-          // forward CTAs retire and run their set-up (TMEM allocation, barrier init, first weight units through TMA) under the forward's tail
-          // (ray compositing, the last CTA's loss seeds / peer exchange); `griddepcontrol.wait` in front of the first read of a forward
-          // result holds them until the forward grid has completed and flushed.
-          cudaLaunchConfig_t cfg; memset(&cfg, 0, sizeof(cfg));
-          cfg.gridDim = dim3((unsigned)grid_t); cfg.blockDim = dim3(tl::kThreads); cfg.dynamicSmemBytes = tile_smem_bytes(true); cfg.stream = st;
-          cudaLaunchAttribute at[1];
-          at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization; at[0].val.programmaticStreamSerializationAllowed = 1;
-          cfg.attrs = at; cfg.numAttrs = 1;
-          if ((rc = check_cuda(cudaLaunchKernelEx(&cfg, render_bwd_tile_kernel, T), "render_bwd_tile_kernel launch (dependent)"))) return rc;
-        } else {
-          render_bwd_tile_kernel<<<(unsigned)grid_t, tl::kThreads, tile_smem_bytes(true), st>>>(T);
-          if ((rc = check_cuda(cudaGetLastError(), "render_bwd_tile_kernel launch"))) return rc;
-        }
-      } else {
-      if (tail != nullptr && tail->px.world > 1) {
+      TileWs w;
+      if (!tile_ws_plan(bw->split_workspace, bw->split_workspace_bytes, in->n_rays, T.S, T.n_dec, true, &w)) {
+        set_error("split_workspace missing or smaller than nsb_split_workspace_bytes(%d, %d)", in->n_rays, T.S); return NSB_ERR_ARG; }
+      T.split = w.split; T.ray_cnt = w.ray_cnt; T.ray_parts = static_cast<double*>(w.scratch); T.tile_rays = tile_rays(T.S);
+      if (sharded) {
         if (n_w != 0 || T.bw.pose_dirs == nullptr) { set_error("sharded backward tail needs pose_dirs and no decoder weight gradients"); return NSB_ERR_ARG; }
         T.tail = *tail;
       }
-      choose_config(in->n_rays, T.S, kRowsBwd, true, T.wbytes, 8, &T, &warps, &smem, kMaxPtsTc);
-      plan_split(&T, T.n_dec, bw->split_workspace, bw->split_workspace_bytes);
-      const int grid_tc = ((in->n_rays + T.rays_per_block - 1) / T.rays_per_block) * T.split;
-      const size_t smem_tc = tc_total_smem(T.max_pts, T.max_rays, true);
-      if (smem_tc > kSmemCap) { set_error("shared-memory budget exceeded (%zu bytes)", smem_tc); return NSB_ERR_UNSUPPORTED; }
-      render_bwd_tc_kernel<<<grid_tc, tc::kThreads, smem_tc, st>>>(T);
-      if ((rc = check_cuda(cudaGetLastError(), "render_bwd_tc_kernel launch"))) return rc;
-      }
+      const long long grid_t = tile_count((long long)in->n_rays * T.S) * T.split;
+      render_bwd_tile_kernel<<<(unsigned)grid_t, tl::kThreads, tile_smem_bytes(true), st>>>(T);
+      if ((rc = check_cuda(cudaGetLastError(), "render_bwd_tile_kernel launch"))) return rc;
       if (n_w == 0) return NSB_OK;
       K.accumulate_rays = 1;
     }

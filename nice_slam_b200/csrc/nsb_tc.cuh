@@ -1,20 +1,11 @@
-// nsb_tc.cuh -- tensor-core evaluation of the NICE decoders: tcgen05.mma (kind::tf32) with a 3xTF32 operand split,
-// accumulators in TMEM.  Included by nsb_render.cu (it uses that file's KParams / Smem / gather helpers).
+// nsb_tc.cuh -- tcgen05 primitives of the tensor-core tile kernels (nsb_tile.cuh): the 3xTF32 operand split, canonical-tile addressing,
+// shared-memory descriptors and the kind::tf32 MMA, plus the optional phase-timing counters.
 //
 // Why 3xTF32: plain TF32 operands miss the 1e-4 parity bar by an order of magnitude (probe: 3e-4 relative on a single
 // 32-wide GEMM); splitting every operand into hi = the 19 bits the tensor core reads, lo = x - hi (exact) and issuing
 // lo*hi + hi*lo + hi*hi gives fp32-level results (probe_tcgen05.cu: 6e-6 abs on |ref| <= 20, same as an FP32 FMA chain).
 //
-// Tile = 128 sample points = 128 TMEM lanes, four threads per point (512-thread CTA).  Activations live in shared memory in the
-// canonical K-major no-swizzle UMMA layout  [row/8][k/4][row%8][k%4]  (core matrix = 8 rows x 16 B): the threads of row r write
-// 16-byte chunks that land conflict-free.  Weights are never touched by threads: nsb_pack_decoders stores every MMA B operand
-// pre-split in that same layout (operand images, nsb_common.cuh) and one elected thread streams the chunks into fixed shared-memory
-// regions with TMA bulk copies, one mbarrier per region, at least one consumer step ahead.
-// Forward per decoder and tile:   gather -> C tile -> D2[128 x 160] = C * [Wc_0..Wc_4]^T (one N = 160 MMA group, not waited for)
-//   -> three embedding blocks E_b, each computed while the previous block's MMAs run: [D1 | D3] += E_b * [W0_b; W3E_b]^T (N = 64)
-//   -> layers 1..4: epilogue h = relu(D + b) + D2_i + bc -> H tile -> D = H * W_i^T (N = 32) -> output layer in registers.
-// Backward (input gradients; the forward saved the ReLU sign bits, nothing is recomputed): per layer one MMA batch
-//   {DC += G * Wc_i, g_i = DU * W_i, DF += DU * W_i^E} from the transposed operand image, two 48 KB stages, layer i-2 in flight.
+// Operand tiles live in shared memory in the canonical K-major no-swizzle UMMA layout  [row/8][k/4][row%8][k%4]  (core matrix = 8 rows x 16 B).
 #pragma once
 
 namespace nsb {
@@ -33,13 +24,6 @@ __device__ long long g_phase_last;
 #endif
 
 constexpr int TM = 128;                 // points per tile
-constexpr uint32_t kTmemCols = 256;     // D1: [0,32)  D2: [32,192)
-// Four threads per point: thread tid owns row (tid & 127) and the 8-column group cg = tid >> 7 of every 32-wide epilogue.
-// Warp w may only touch TMEM lanes [32 (w & 3), +32): with this numbering the row of a thread is exactly such a lane.
-constexpr int kThreads = 512;
-constexpr int kCG = kThreads / TM;      // column groups (threads per point)
-constexpr int kCW = 32 / kCG;           // columns per thread
-constexpr int kKQ = kCW / 4;            // 16-byte operand chunks per thread and 32-wide tile row
 
 // hi part of the 3xTF32 split: the top 19 bits (sign, exponent, 10 mantissa bits) -- exactly what the tensor core reads of
 // an fp32 word.  Truncation instead of cvt.rna keeps x = hi + lo exact (lo has <= 13 significant bits, of which the MMA
@@ -81,497 +65,11 @@ __device__ __forceinline__ uint32_t elect_one() {
   asm volatile("{\n\t.reg .pred q;\n\telect.sync _|q, 0xffffffff;\n\tselp.b32 %0, 1, 0, q;\n\t}" : "=r"(p) :: "memory");
   return p;
 }
-// D[128 x N] (+)= A[128 x kcount*8] * B[N x kcount*8]^T with the 3xTF32 split.  Called by all lanes of warp 0.  A/B tiles have widths KA/KB floats and
-// the product starts at column ka0 / kb0 (multiples of 8).  `acc` is the running accumulate flag of this D.
-__device__ __forceinline__ void mma_3x(uint32_t d_tmem, const float* a_hi, const float* a_lo, int KA, int ka0,
-                                       const float* b_hi, const float* b_lo, int KB, int kb0, int kcount, int N, uint32_t& acc) {
-  const uint32_t idesc = make_idesc(TM, N);
-  const uint32_t sboA = (uint32_t)(KA >> 2) * 128u, sboB = (uint32_t)(KB >> 2) * 128u;
-  const uint64_t ah0 = make_desc(a_hi + (ka0 >> 2) * 32, 128u, sboA), al0 = make_desc(a_lo + (ka0 >> 2) * 32, 128u, sboA);
-  const uint64_t bh0 = make_desc(b_hi + (kb0 >> 2) * 32, 128u, sboB), bl0 = make_desc(b_lo + (kb0 >> 2) * 32, 128u, sboB);
-  if (elect_one()) {
-    for (int ks = 0; ks < kcount; ks++) {                      // one k-step of 8 floats = two core matrices = +16 in the 16-byte-granular address field
-      const uint64_t o = 16u * (uint64_t)ks;
-      mma_tf32(d_tmem, al0 + o, bh0 + o, idesc, ks == 0 ? acc : 1u);
-      mma_tf32(d_tmem, ah0 + o, bl0 + o, idesc, 1u);
-      mma_tf32(d_tmem, ah0 + o, bh0 + o, idesc, 1u);
-    }
-  }
-  __syncwarp();
-  acc = 1u;
-}
-__device__ __forceinline__ void mma_commit_elect(uint64_t* bar) {
-  if (elect_one()) asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-  __syncwarp();
-}
 __device__ __forceinline__ void mma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-// operands written by this thread (generic proxy) -> visible to the tensor core (async proxy), then CTA barrier
-__device__ __forceinline__ void publish_operands() { fence_proxy_async(); tc_fence_before(); __syncthreads(); }
-
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, float (&v)[32]) {
-  uint32_t r[32];
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-               "{%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]), "=r"(r[10]),
-                 "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]), "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]),
-                 "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-               : "r"(taddr) : "memory");
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-  for (int j = 0; j < 32; j++) v[j] = __uint_as_float(r[j]);
-}
-
-__device__ __forceinline__ void tmem_ld8(uint32_t taddr, float (&v)[8]) {
-  uint32_t r[8];
-  asm volatile("tcgen05.ld.sync.aligned.32x32b.x8.b32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-               : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]) : "r"(taddr) : "memory");
-  asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-  for (int j = 0; j < 8; j++) v[j] = __uint_as_float(r[j]);
-}
-static_assert(kCW == 8, "epilogues use tcgen05.ld.32x32b.x8");
-
-// ---- shared memory and barriers of the tensor-core kernels ---------------------------------------------------------------------
-// Weights are never staged by threads: nsb_pack_decoders leaves every MMA B operand as a ready-to-use hi|lo canonical tile in global
-// memory (operand images, nsb_common.cuh) and one elected thread streams them into fixed shared-memory regions with TMA bulk copies,
-// one mbarrier per region, always at least one consumer step ahead of the MMAs that read them.
-struct TcSmem {
-  float* x;          // 64 KB activation tiles: C hi|lo (128 x cd)  -> later E block 1 (first 32 KB) and H (second 32 KB); backward: G | DU, then dL/dc
-  float* e;          // forward: 32 KB E blocks 0 and 2, later the output-layer partial sums
-  float* wF;         // forward: fc_c chunk (40 KB)
-  float* wL;         // forward: two layer-0 chunks (2 x 16 KB)
-  float* wH;         // forward: hidden weights of layers 1..4 (32 KB)
-  float* wS;         // backward: two layer stages (2 x 48 KB)
-  float* hdr;        // 2 x kHdrFloats: biases, output weights, embedding matrix (double-buffered over decoders)
-  uint64_t* bars;    // mbarriers (see the B_* indices)
-  uint32_t* tmem;    // TMEM base address slot
-};
-constexpr int kXFloats = 2 * TM * 64;            // 16384 floats = 64 KB
-constexpr int kEFloats = 2 * TM * 32;            // 32 KB
-// barrier indices.  forward: TMA arrivals W_*, MMA commits M_*; backward reuses W_HDR, W_S0/1 and M_B.
-enum { W_HDR = 0, W_F, W_L0, W_L1, W_H, M_FC, M_L0, M_L1, M_H, kNumBarsFwd, W_S0 = 1, W_S1 = 2, M_B = 3, kNumBarsBwd = 4 };
-__host__ __device__ inline size_t tc_smem_bytes(bool bwd) {
-  const size_t fl = bwd ? (size_t)kXFloats + 2 * kBwdStageFloats + 2 * kHdrFloats
-                        : (size_t)kXFloats + kEFloats + kFcChunk + 2 * kL0Chunk + 4 * kHChunk + 2 * kHdrFloats;
-  return fl * 4 + 128;
-}
-__device__ __forceinline__ void tc_carve(unsigned char* base, TcSmem& t, bool bwd) {
-  float* f = reinterpret_cast<float*>(base);
-  t.x = f; f += kXFloats;
-  t.e = t.wF = t.wL = t.wH = t.wS = nullptr;
-  if (bwd) { t.wS = f; f += 2 * kBwdStageFloats; }
-  else { t.e = f; f += kEFloats; t.wF = f; f += kFcChunk; t.wL = f; f += 2 * kL0Chunk; t.wH = f; f += 4 * kHChunk; }
-  t.hdr = f; f += 2 * kHdrFloats;
-  t.bars = reinterpret_cast<uint64_t*>(f);
-  t.tmem = reinterpret_cast<uint32_t*>(f + 2 * 12);
-}
-// running state of the weight pipeline, identical in every thread (control flow is CTA-uniform)
-struct Pipe {
-  uint32_t par;          // bit i = parity the next wait on barrier i expects
-  int hb;                // header buffer of the current decoder
-  bool prefetched;       // the current decoder's first loads are already in flight
-};
-__device__ __forceinline__ void pipe_wait(const TcSmem& t, Pipe& p, int i, bool really = true) {
-  if (really) mbar_wait(t.bars + i, (p.par >> i) & 1u);
-  p.par ^= 1u << i;
-}
-// one elected thread: bulk copy `floats` floats, completion on barrier i
-__device__ __forceinline__ void tma_load(const TcSmem& t, int i, float* dst, const float* src, int floats) {
-  const uint32_t bytes = (uint32_t)floats * 4u;
-  mbar_expect_tx(t.bars + i, bytes);
-  for (uint32_t off = 0; off < bytes; off += 32768u)
-    tma_bulk_g2s(reinterpret_cast<char*>(dst) + off, reinterpret_cast<const char*>(src) + off, bytes - off < 32768u ? bytes - off : 32768u, t.bars + i);
-}
-// first loads of decoder lv (forward): header, first fc_c chunk, first two layer-0 chunks, hidden weights
-__device__ __forceinline__ void issue_fwd_loads(const KParams& P, const TcSmem& t, int lv, int hb) {
-  const float* img = P.in.packed[lv] + op_fwd_offset(lv);
-  tma_load(t, W_HDR, t.hdr + hb * kHdrFloats, img, kHdrFloats);
-  const float* fc = img + kHdrFloats;
-  if (lv != 0) tma_load(t, W_F, t.wF, fc, kFcChunk);
-  const float* l0 = fc + op_fc_floats(lv);
-  tma_load(t, W_L0, t.wL, l0, kL0Chunk);
-  if (lv != 0) tma_load(t, W_L1, t.wL + kL0Chunk, l0 + kL0Chunk, kL0Chunk);
-  tma_load(t, W_H, t.wH, l0 + op_nblk(lv) * kL0Chunk, 4 * kHChunk);
-}
-// first loads of decoder lv (backward): header, layers 4 and 3
-__device__ __forceinline__ void issue_bwd_loads(const KParams& P, const TcSmem& t, int lv, int hb) {
-  tma_load(t, W_HDR, t.hdr + hb * kHdrFloats, P.in.packed[lv] + op_fwd_offset(lv), kHdrFloats);
-  const float* img = P.in.packed[lv] + op_bwd_offset(lv);
-  tma_load(t, W_S0, t.wS, img + op_bwd_layer_offset(lv, 4), op_bwd_layer_floats(lv, 4));
-  tma_load(t, W_S1, t.wS + kBwdStageFloats, img + op_bwd_layer_offset(lv, 3), op_bwd_layer_floats(lv, 3));
-}
-
-// 8 lanes per point, 4 points per pass: gather the 32 channels of `g` into columns [col0, col0+32) of the C tile.  Warp w serves
-// the rows of its lane quadrant (w & 3); the eight passes of a quadrant are split over the kCG warps that share it.
-__device__ __forceinline__ void gather_rows(const nsb_grid& g, float* c_hi, float* c_lo, int KC, int col0,
-                                            const float xn[3], int warp, int lane) {
-  const bool fast = grid_fast(g);
-  const int q = lane & 7, qd = warp & 3, it0 = (warp >> 2) * (8 / kCG);
-  static_assert(8 / kCG == 2, "one batch of two passes per warp");
-  Tri t[2]; float4 v[2][8];                                        // 16 loads in flight per lane
-#pragma unroll
-  for (int u = 0; u < 2; u++) {
-    const int src_lane = (it0 + u) * 4 + (lane >> 3);
-    float x[3];
-    x[0] = __shfl_sync(0xffffffffu, xn[0], src_lane); x[1] = __shfl_sync(0xffffffffu, xn[1], src_lane); x[2] = __shfl_sync(0xffffffffu, xn[2], src_lane);
-    t[u] = make_tri(x, g.W, g.H, g.D);
-#pragma unroll
-    for (int k = 0; k < 8; k++) {
-      int cx, cy, cz;
-      tri_corner_clamped(t[u], k, g.W, g.H, g.D, cx, cy, cz);
-      v[u][k] = grid_load4(g, cz * g.stride_d + cy * g.stride_h + cx * g.stride_w, 4 * q, fast);
-    }
-  }
-#pragma unroll
-  for (int u = 0; u < 2; u++) {
-    float4 acc = make_float4(0.f, 0.f, 0.f, 0.f);
-#pragma unroll
-    for (int k = 0; k < 8; k++) {
-      const float w = tri_weight(t[u], k);
-      acc.x = fmaf(v[u][k].x, w, acc.x); acc.y = fmaf(v[u][k].y, w, acc.y); acc.z = fmaf(v[u][k].z, w, acc.z); acc.w = fmaf(v[u][k].w, w, acc.w);
-    }
-    put4(c_hi, c_lo, qd * 32 + (it0 + u) * 4 + (lane >> 3), (col0 >> 2) + q, KC, acc);
-  }
-}
-
-// this thread's kCW features of E block `blk` (features 32*blk .. +31, zero beyond 93) of its point -> canonical hi|lo tile of width 32
-__device__ __forceinline__ void embed_row(float* e_hi, float* e_lo, const float* B /*packed [3][96]*/,
-                                          const float pf[3], int row, int cg, int blk) {
-#pragma unroll
-  for (int kq = kKQ * cg; kq < kKQ * cg + kKQ; kq++) {
-    float v[4];
-#pragma unroll
-    for (int j = 0; j < 4; j++) {
-      const int f = 32 * blk + 4 * kq + j;
-      float x = pf[0] * B[f]; x = fmaf(pf[1], B[kEmbPad + f], x); x = fmaf(pf[2], B[2 * kEmbPad + f], x);
-      v[j] = f < kEmb ? __sinf(reduce_2pi(x)) : 0.0f;
-    }
-    put4(e_hi, e_lo, row, kq, 32, make_float4(v[0], v[1], v[2], v[3]));
-  }
-}
-
-// Forward of decoder `lv` for one 128-point tile.  Thread tid = (row = tid & 127, column group cg = tid >> 7).  On return out[o] holds
-// the decoder outputs of this thread's point (identical in the kCG threads of a row).
-// TMEM: D1 = cols [0,32) (layers 0,1,2,4), D3 = [32,64) (layer 3; its skip part E * W3E^T is accumulated while the embedding blocks are
-// live for layer 0, so the embedding is computed once, by one N = 64 MMA per block), D2 = [64,224) (fc_c of the five layers, one N = 160 MMA).
-// Step order (xyz decoder):  gather C | fc_c MMAs (async) | E0 -> MMA | wait fc_c | E1 -> MMA | wait E0 | E2 -> MMA | five serial
-// epilogue -> MMA steps.  Each embedding block is computed while the previous block's MMAs run.
-__device__ __forceinline__ void tile_forward(const KParams& P, const TcSmem& t, const DecRT& d, int lv, const PointGeom& G,
-                                             uint32_t tmem, Pipe& pp, float (&out)[4],
-                                             uint32_t* __restrict__ gmask /* global [5] slot of this point+decoder, or nullptr */,
-                                             int next_lv /* decoder whose weights to prefetch once this one's regions are free, or -1 */) {
-  const int row = threadIdx.x & (TM - 1), cg = threadIdx.x >> 7, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const bool t0 = threadIdx.x == 0, w0 = threadIdx.x < 32;
-  const uint32_t my = ((uint32_t)((warp & 3) * 32) << 16) + (uint32_t)(kCW * cg);      // TMEM lane quadrant + first column of this thread
-  const uint32_t d1 = tmem + my, d3 = tmem + 32u + my, d2 = tmem + 64u + my;
-  const float* hdr = t.hdr + pp.hb * kHdrFloats;
-  float* c_hi = t.x; float* c_lo = t.x + TM * d.cd;
-
-  __syncthreads();                       // previous decoder / tile: every read of x, e and of the header buffers is done
-  NSB_PH(0);
-  if (!pp.prefetched && t0) issue_fwd_loads(P, t, lv, pp.hb);
-  pp.prefetched = false;
-  // ---- gather -> C tile
-  const float* xn = lv == 0 ? G.xnc : G.xn;
-  gather_rows(P.in.grid[lv], c_hi, c_lo, d.cd, 0, xn, warp, lane);
-  if (lv == 2) gather_rows(P.in.grid[1], c_hi, c_lo, d.cd, 32, G.xn, warp, lane);
-  NSB_PH(1);
-  // ---- D2 = C * [Wc_0; ..; Wc_4]^T  (xyz decoders), one 32-wide K half per chunk; not waited for until x is needed again
-  if (d.xyz) {
-    publish_operands();
-    for (int h = 0; h < (d.cd >> 5); h++) {
-      if (w0) {
-        if (h > 0) { mbar_wait(t.bars + M_FC, (pp.par >> M_FC) & 1u);          // chunk 0 consumed: reload the region with chunk 1
-                     if (t0) tma_load(t, W_F, t.wF, P.in.packed[lv] + op_fwd_offset(lv) + kHdrFloats + kFcChunk, kFcChunk);
-                     __syncwarp(); }
-        mbar_wait(t.bars + W_F, (pp.par >> W_F) & 1u);
-        tc_fence_after();
-        uint32_t acc = h > 0 ? 1u : 0u;
-        mma_3x(tmem + 64u, c_hi, c_lo, d.cd, 32 * h, t.wF, t.wF + 160 * 32, 32, 0, 4, 160, acc);
-        mma_commit_elect(t.bars + M_FC);
-      }
-      pp.par ^= 1u << W_F;
-      if (h > 0) pp.par ^= 1u << M_FC;
-      __syncwarp();
-    }
-  }
-  NSB_PH(2);
-  // ---- layer 0 and the skip part of layer 3: [D1 | D3] += E_blk * [W0_blk; W3E_blk]^T.  E = Fourier embedding, or (coarse) C itself.
-  const float* B = hdr + 464;
-  const int nblk = d.xyz ? 3 : 1;
-  bool fc_pending = d.xyz != 0;
-  for (int blk = 0; blk < nblk; blk++) {
-    float* e_hi = !d.xyz ? c_hi : ((blk & 1) ? t.x : t.e);
-    float* e_lo = !d.xyz ? c_lo : e_hi + TM * 32;
-    if (d.xyz) {
-      if (blk == 0) pipe_wait(t, pp, W_HDR);                                   // embedding matrix
-      if (blk == 1) { pipe_wait(t, pp, M_FC); fc_pending = false; tc_fence_after(); }      // C is dead: x may be overwritten
-      if (blk == 2) {                                                          // block 0 consumed: e and weight slot 0 are free
-        pipe_wait(t, pp, M_L0); tc_fence_after();
-        if (t0) tma_load(t, W_L0, t.wL, P.in.packed[lv] + op_fwd_offset(lv) + kHdrFloats + op_fc_floats(lv) + 2 * kL0Chunk, kL0Chunk);
-      }
-      embed_row(e_hi, e_lo, B, G.pf, row, cg, blk);
-    }
-    publish_operands();
-    const int slot = blk & 1;
-    if (w0) {
-      mbar_wait(t.bars + W_L0 + slot, (pp.par >> (W_L0 + slot)) & 1u);
-      tc_fence_after();
-      uint32_t acc = blk > 0 ? 1u : 0u;
-      const float* w = t.wL + slot * kL0Chunk;
-      mma_3x(tmem, e_hi, e_lo, 32, 0, w, w + 64 * 32, 32, 0, 4, 64, acc);
-      mma_commit_elect(t.bars + M_L0 + slot);
-    }
-    pp.par ^= 1u << (W_L0 + slot);
-    __syncwarp();
-    NSB_PH(3 + blk);
-  }
-  if (!d.xyz) pipe_wait(t, pp, W_HDR);
-  if (fc_pending) pipe_wait(t, pp, M_FC);
-  if (nblk > 1) pipe_wait(t, pp, M_L1);
-  pipe_wait(t, pp, M_L0);                                   // (blocks 0/2 use slot 0: the last commit on it is block nblk-1 or 2)
-  tc_fence_after();
-  NSB_PH(6);
-  float* h_hi = t.x + 2 * TM * 32;
-  float* h_lo = t.x + 3 * TM * 32;
-  float h[kCW];
-#pragma unroll 1
-  for (int i = 0; i < 5; i++) {
-    // ---- epilogue of layer i (this thread's kCW columns): h = relu(D + b_i) + (D2_i + bc_i)
-    float v1[kCW];
-    tmem_ld8(i == 3 ? d3 : d1, v1);
-    uint32_t m = 0;
-#pragma unroll
-    for (int j = 0; j < kCW; j++) { const float u = v1[j] + hdr[i * 32 + kCW * cg + j]; h[j] = u > 0.0f ? u : 0.0f; m |= u > 0.0f ? (1u << j) : 0u; }
-    if (gmask != nullptr) reinterpret_cast<uint8_t*>(gmask)[i * 4 + cg] = (uint8_t)m;      // byte cg of the 32-bit ReLU mask word
-    if (d.xyz) {
-      float v2[kCW];
-      tmem_ld8(d2 + 32u * i, v2);
-#pragma unroll
-      for (int j = 0; j < kCW; j++) h[j] += v2[j] + hdr[160 + i * 32 + kCW * cg + j];
-    }
-    if (i == 4) break;
-#pragma unroll
-    for (int k = 0; k < kKQ; k++) put4(h_hi, h_lo, row, kKQ * cg + k, 32, make_float4(h[4 * k], h[4 * k + 1], h[4 * k + 2], h[4 * k + 3]));
-    publish_operands();                                      // (also orders this layer's TMEM reads before the next MMAs)
-    if (w0) {
-      if (i == 0) mbar_wait(t.bars + W_H, (pp.par >> W_H) & 1u);
-      tc_fence_after();
-      const float* w = t.wH + i * kHChunk;                   // hidden weights of layer i+1
-      uint32_t acc = (i + 1 == 3) ? 1u : 0u;                 // layer 3 accumulates onto E * W3E^T
-      mma_3x((i + 1 == 3) ? tmem + 32u : tmem, h_hi, h_lo, 32, 0, w, w + 32 * 32, 32, 0, 4, 32, acc);
-      mma_commit_elect(t.bars + M_H);
-    }
-    if (i == 0) pp.par ^= 1u << W_H;
-    __syncwarp();
-    pipe_wait(t, pp, M_H);
-    tc_fence_after();
-    NSB_PH(7 + i);
-  }
-  tc_fence_before();
-  // every weight region is free again: prefetch the next decoder's first chunks under the output layer and the next gather
-  if (next_lv >= 0) { if (t0) issue_fwd_loads(P, t, next_lv, pp.hb ^ 1); pp.prefetched = true; }
-  // ---- output layer: partial dot products over this thread's columns, summed over the kCG threads of the row through shared memory
-  float* part = d.xyz ? t.e : t.x;                           // [kCG][TM][4]   (E blocks / the coarse C tile are dead)
-  {
-    float s[4];
-#pragma unroll
-    for (int o = 0; o < 4; o++) {
-      s[o] = 0.0f;
-      if (o < d.no) {
-#pragma unroll
-        for (int j = 0; j < kCW; j++) s[o] = fmaf(h[j], hdr[336 + o * 32 + kCW * cg + j], s[o]);
-      }
-    }
-    *reinterpret_cast<float4*>(part + (cg * TM + row) * 4) = make_float4(s[0], s[1], s[2], s[3]);
-  }
-  __syncthreads();
-#pragma unroll
-  for (int o = 0; o < 4; o++) out[o] = hdr[320 + o];
-#pragma unroll
-  for (int c = 0; c < kCG; c++) {
-    const float4 v = *reinterpret_cast<const float4*>(part + (c * TM + row) * 4);
-    out[0] += v.x; out[1] += v.y; out[2] += v.z; out[3] += v.w;
-  }
-  pp.hb ^= 1;
-  NSB_PH(12);
-}
-
-// Backward of decoder `lv` for one tile, input gradients only (rays + grid voxels; decoder-weight gradients go through the FP32 kernel).
-// gmask = the ReLU masks the forward kernel saved for this point+decoder.  g_out = dL/d out of this thread's point.
-// Writes dL/dc of every row to `dcs` ([128][cd] fp32, aliasing t.x) and this thread's share of dL/dp through the Fourier embedding to
-// [kCG][128][4] fp32 at t.x + 2*TM*32 (summed by the caller after a barrier: dpe_sum).
-// TMEM: D1 = [0,32) (g of the next layer), DC = [32,96) (dL/dc, accumulated over the layers), DF = [96,192) (dL/d first input).
-// One MMA batch per layer; the operands of layer i-2 are fetched by TMA while layer i computes (two 48 KB stages).
-__device__ __forceinline__ void tile_backward(const KParams& P, const TcSmem& t, const DecRT& d, int lv, const PointGeom& G,
-                                              uint32_t tmem, Pipe& pp, const float (&g_out)[4], const uint32_t* __restrict__ gmask,
-                                              int next_lv) {
-  const int row = threadIdx.x & (TM - 1), cg = threadIdx.x >> 7, warp = threadIdx.x >> 5;
-  const bool t0 = threadIdx.x == 0, w0 = threadIdx.x < 32;
-  const float* hdr = t.hdr + pp.hb * kHdrFloats;
-  __syncthreads();                                          // previous decoder's scatter (reads of x) is done
-  NSB_PH(20);
-  if (!pp.prefetched && t0) issue_bwd_loads(P, t, lv, pp.hb);
-  pp.prefetched = false;
-  uint32_t mlo = 0, mhi = 0;                                // this thread's 8 ReLU bits of layers 0..3 (one byte each) and of layer 4
-#pragma unroll
-  for (int i = 0; i < 4; i++) mlo |= (uint32_t) reinterpret_cast<const uint8_t*>(gmask)[i * 4 + cg] << (8 * i);
-  mhi = reinterpret_cast<const uint8_t*>(gmask)[16 + cg];
-  pipe_wait(t, pp, W_HDR);
-  const uint32_t my = ((uint32_t)((warp & 3) * 32) << 16) + (uint32_t)(kCW * cg);
-  const uint32_t dcc = tmem + 32u, dfc = tmem + 96u;
-  float* g_hi = t.x; float* g_lo = t.x + TM * 32;
-  float* du_hi = t.x + 2 * TM * 32; float* du_lo = t.x + 3 * TM * 32;
-  float g[kCW];
-#pragma unroll
-  for (int j = 0; j < kCW; j++) {
-    float v = 0.0f;
-#pragma unroll
-    for (int o = 0; o < 4; o++) v = fmaf(hdr[336 + o * 32 + kCW * cg + j], g_out[o], v);       // rows >= NO are zero
-    g[j] = v;
-  }
-  uint32_t acc_dc = 0, acc_df = 0;
-  const float* img = P.in.packed[lv] + op_bwd_offset(lv);
-  NSB_PH(21);
-#pragma unroll 1
-  for (int i = 4; i >= 0; i--) {
-    const uint32_t m = i == 4 ? mhi : (mlo >> (8 * i)) & 0xffu;
-    const int s = (4 - i) & 1;                               // stage of this layer's operands
-#pragma unroll
-    for (int k = 0; k < kKQ; k++) {
-      if (d.xyz) put4(g_hi, g_lo, row, kKQ * cg + k, 32, make_float4(g[4 * k], g[4 * k + 1], g[4 * k + 2], g[4 * k + 3]));
-      put4(du_hi, du_lo, row, kKQ * cg + k, 32, make_float4((m >> (4 * k)) & 1u ? g[4 * k] : 0.0f, (m >> (4 * k + 1)) & 1u ? g[4 * k + 1] : 0.0f,
-                                                             (m >> (4 * k + 2)) & 1u ? g[4 * k + 2] : 0.0f, (m >> (4 * k + 3)) & 1u ? g[4 * k + 3] : 0.0f));
-    }
-    publish_operands();
-    if (w0) {   // DC += G * Wc_i (dL/dc through fc_c) ; D1 = DU * W_i[:, hidden] (g_i) ; DF += DU * W_i[:, first] (i = 3, 0)
-      mbar_wait(t.bars + W_S0 + s, (pp.par >> (W_S0 + s)) & 1u);
-      tc_fence_after();
-      const float* w = t.wS + s * kBwdStageFloats;
-      if (d.xyz) { mma_3x(dcc, g_hi, g_lo, 32, 0, w, w + d.cd * 32, 32, 0, 4, d.cd, acc_dc); w += 2 * d.cd * 32; }
-      if (i >= 1) { uint32_t a1 = 0; mma_3x(tmem, du_hi, du_lo, 32, 0, w, w + 32 * 32, 32, 0, 4, 32, a1); w += kHChunk; }
-      if (i == 3 || i == 0) mma_3x(dfc, du_hi, du_lo, 32, 0, w, w + d.firstp * 32, 32, 0, 4, d.firstp, acc_df);
-      mma_commit_elect(t.bars + M_B);
-    }
-    pp.par ^= 1u << (W_S0 + s);
-    __syncwarp();
-    pipe_wait(t, pp, M_B);
-    tc_fence_after();
-    if (t0 && i >= 2) tma_load(t, W_S0 + s, t.wS + s * kBwdStageFloats, img + op_bwd_layer_offset(lv, i - 2), op_bwd_layer_floats(lv, i - 2));
-    if (i >= 1) tmem_ld8(tmem + my, g);
-    tc_fence_before();
-    NSB_PH(22 + (4 - i));
-  }
-  // both stages are free: the next decoder's header and first two layers arrive under the epilogue and the scatter
-  if (next_lv >= 0) { if (t0) issue_bwd_loads(P, t, next_lv, pp.hb ^ 1); pp.prefetched = true; }
-  // ---- dL/dc rows -> shared (plain fp32 [128][cd]); all MMAs reading t.x have completed
-  float* dcs = t.x;
-  {
-    float v[kCW];
-    const int nch = d.xyz ? (d.cd >> 5) : 1;
-    for (int c = 0; c < nch; c++) {
-      tmem_ld8((d.xyz ? dcc : dfc) + 32u * c + my, v);
-#pragma unroll
-      for (int k = 0; k < kKQ; k++)
-        *reinterpret_cast<float4*>(dcs + row * d.cd + 32 * c + kCW * cg + 4 * k) = make_float4(v[4 * k], v[4 * k + 1], v[4 * k + 2], v[4 * k + 3]);
-    }
-  }
-  // ---- embedding chain: dp += B (cos(pB) * dfirst), this thread's features; partial sums to shared memory
-  float dpe[3] = {0.0f, 0.0f, 0.0f};
-  if (d.xyz) {
-    const float* B = hdr + 464;
-    for (int c = 0; c < 3; c++) {
-      float v[kCW];
-      tmem_ld8(dfc + 32u * c + my, v);
-#pragma unroll
-      for (int j = 0; j < kCW; j++) {
-        const int f = 32 * c + kCW * cg + j;
-        if (f < kEmb) {
-          const float b0 = B[f], b1 = B[kEmbPad + f], b2 = B[2 * kEmbPad + f];
-          float x = G.pf[0] * b0; x = fmaf(G.pf[1], b1, x); x = fmaf(G.pf[2], b2, x);
-          const float dx = __cosf(reduce_2pi(x)) * v[j];
-          dpe[0] = fmaf(b0, dx, dpe[0]); dpe[1] = fmaf(b1, dx, dpe[1]); dpe[2] = fmaf(b2, dx, dpe[2]);
-        }
-      }
-    }
-  }
-  *reinterpret_cast<float4*>(t.x + 2 * TM * 32 + (cg * TM + row) * 4) = make_float4(dpe[0], dpe[1], dpe[2], 0.0f);
-  tc_fence_before();
-  pp.hb ^= 1;
-  NSB_PH(27);
-}
-// dL/dp of `row` through the embedding: sum of the kCG partials tile_backward left in shared memory (call after a CTA barrier)
-__device__ __forceinline__ void dpe_sum(const TcSmem& t, int row, float (&dpe)[3]) {
-  dpe[0] = dpe[1] = dpe[2] = 0.0f;
-#pragma unroll
-  for (int c = 0; c < kCG; c++) {
-    const float4 v = *reinterpret_cast<const float4*>(t.x + 2 * TM * 32 + (c * TM + row) * 4);
-    dpe[0] += v.x; dpe[1] += v.y; dpe[2] += v.z;
-  }
-}
-
-// Backward of gather_rows (same warp -> rows mapping): dc rows come from `dcs` ([128][cd] fp32).  Scatter-adds into dgrid (if non-null)
-// and hands the normalised-coordinate gradient of each point to emit(row, gx).
-template <typename F>
-__device__ __forceinline__ void scatter_rows(const nsb_grid& g, float* __restrict__ dgrid, const int32_t* __restrict__ slots,
-                                             const float* dcs, int cd,
-                                             const float xn[3], int warp, int lane, F&& emit) {
-  const bool fast = grid_fast(g);
-  const int q = lane & 7, qd = warp & 3, it0 = (warp >> 2) * (8 / kCG);
-#pragma unroll 1
-  for (int it = it0; it < it0 + 8 / kCG; it++) {
-    const int src_lane = it * 4 + (lane >> 3);
-    const int row = qd * 32 + src_lane;
-    float x[3];
-    x[0] = __shfl_sync(0xffffffffu, xn[0], src_lane); x[1] = __shfl_sync(0xffffffffu, xn[1], src_lane); x[2] = __shfl_sync(0xffffffffu, xn[2], src_lane);
-    const Tri t = make_tri(x, g.W, g.H, g.D);
-    const float4 d4 = *reinterpret_cast<const float4*>(dcs + row * cd + 4 * q);
-    const float dc[4] = {d4.x, d4.y, d4.z, d4.w};
-    float gi[3] = {0.f, 0.f, 0.f};
-    long long offs[8]; float4 vv[8]; bool ins[8];
-#pragma unroll
-    for (int k = 0; k < 8; k++) {                                // all corner loads first (branch-free clamped addressing)
-      int cx, cy, cz;
-      ins[k] = tri_corner(t, k, g.W, g.H, g.D, cx, cy, cz);
-      tri_corner_clamped(t, k, g.W, g.H, g.D, cx, cy, cz);
-      offs[k] = cz * g.stride_d + cy * g.stride_h + cx * g.stride_w;
-      vv[k] = grid_load4(g, offs[k], 4 * q, fast);
-    }
-#pragma unroll
-    for (int k = 0; k < 8; k++) {
-      if (ins[k]) {
-        const float4 v = vv[k];
-        const float dot = v.x * dc[0] + v.y * dc[1] + v.z * dc[2] + v.w * dc[3];
-        if (dgrid != nullptr) {
-          int cx, cy, cz;
-          tri_corner(t, k, g.W, g.H, g.D, cx, cy, cz);
-          voxel_grad_add(g, dgrid, slots, offs[k], cx, cy, cz, q, fast, tri_weight(t, k), dc);
-        }
-        const float wx = (k & 1) ? t.w1[0] : t.w0[0], wy = (k & 2) ? t.w1[1] : t.w0[1], wz = (k & 4) ? t.w1[2] : t.w0[2];
-        gi[0] += ((k & 1) ? 1.f : -1.f) * wy * wz * dot;
-        gi[1] += ((k & 2) ? 1.f : -1.f) * wx * wz * dot;
-        gi[2] += ((k & 4) ? 1.f : -1.f) * wx * wy * dot;
-      }
-    }
-#pragma unroll
-    for (int a = 0; a < 3; a++) {
-      float v = gi[a];
-      v += __shfl_xor_sync(0xffffffffu, v, 1); v += __shfl_xor_sync(0xffffffffu, v, 2); v += __shfl_xor_sync(0xffffffffu, v, 4);
-      gi[a] = v;
-    }
-    if (q == 0) {
-      const int size[3] = {g.W, g.H, g.D};
-      float gx[3];
-#pragma unroll
-      for (int a = 0; a < 3; a++) gx[a] = t.clipg[a] * ((float)(size[a] - 1) * 0.5f) * gi[a];
-      emit(row, gx);
-    }
-  }
-}
 
 }  // namespace tc
 }  // namespace nsb

@@ -20,8 +20,7 @@
 // Shared memory: 64 KB activations + 40 KB ring + 6 KB headers + < 6 KB state <= 113 KB, TMEM 256 columns -> two CTAs per SM, i.e. two
 // tiles in flight per SM with the hardware interleaving their (latency-bound) chains.
 //
-// Arithmetic is that of nsb_tc.cuh (3xTF32 split, same operand order), so results match the round-1 kernels to rounding of the output
-// layer's partial sums.
+// Operands are split as nsb_tc.cuh describes (3xTF32: hi = the 19 bits the tensor core reads, lo = x - hi), which gives FP32-level results.
 #pragma once
 
 namespace nsb {
@@ -162,7 +161,7 @@ __device__ __forceinline__ void loader_top_up(Loader& L, const TileSmem& t, uint
 __device__ __forceinline__ void load_header(const KParams& P, const TileSmem& t, int lv, int hb) {
   uint64_t* bar = t.bars + B_HDR + hb;
   mbar_expect_tx(bar, kHdrFloats * 4u);
-  tma_bulk_g2s(t.hdr + hb * kHdrFloats, P.in.packed[lv] + op_fwd_offset(lv), kHdrFloats * 4u, bar);
+  tma_bulk_g2s(t.hdr + hb * kHdrFloats, P.in.packed[lv] + op_hdr_offset(lv), kHdrFloats * 4u, bar);
 }
 
 // Issuer state (control thread)
@@ -1217,9 +1216,6 @@ __device__ __forceinline__ void render_fwd_tile_body(const KParams& P) {
   tc::tc_fence_before();
   __syncthreads();
   if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(kTmemCols) : "memory");
-  // the decoder chain of this item is done: a backward launched as a programmatic dependent may take the slots that free up from here on and
-  // set up under the ray compositing / loss-seed tail (triggering at kernel start made the early backward CTAs compete with the chain: slower)
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
   NSB_PH(14);
 
   if (points) {                                                   // Renderer.eval_points: raw with the out-of-bound override
@@ -1302,9 +1298,6 @@ __device__ __forceinline__ void render_bwd_tile_body(const KParams& P) {
   }
 
   for (int i = tid; i < TM * 3; i += kThreads) X.dp[i] = 0.0;
-  // Launched as a programmatic dependent of the forward (nsb_render.cu): everything above ran under the forward's tail; nothing the forward
-  // produces (raw, z_vals, ReLU bits, loss seeds, completion counters) is touched before the forward grid has completed.  (No-op otherwise.)
-  asm volatile("griddepcontrol.wait;" ::: "memory");
   // ---- prologue: per ray of this tile, compositing weights and dL/d(occupancy logit) (SURVEY.md 8.1); scratch in the operand buffers
   for (int r = warp; r < nr; r += kThreads / 32) {
     const int ray = ray_lo + r;

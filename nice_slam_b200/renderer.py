@@ -176,7 +176,7 @@ class _RenderFn(torch.autograd.Function):
         z_vals = torch.empty(n, S, dtype=torch.float64, device=dev)
         raw = torch.empty(n, S, 4, dtype=torch.float32, device=dev)
         masks = torch.empty(n, S, 15, dtype=torch.int32, device=dev)      # ReLU sign bits: lets backward skip the forward recompute
-        nsplit = L.nsb_split_workspace_bytes(n, S)                        # small batches: one CTA per (ray group, decoder)
+        nsplit = L.nsb_split_workspace_bytes(n, S)                        # tile kernels: ray completion counters + per-item scratch
         split = torch.zeros(nsplit, dtype=torch.uint8, device=dev) if nsplit else None
         # colour-decoder parameters that need a gradient (the mapper's colour stage, Mapper.py:339-341): keep the decoder's layer outputs so that
         # the backward computes the weight gradients on the tensor cores

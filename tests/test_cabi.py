@@ -160,3 +160,22 @@ def test_iteration_context_block_layouts_on_cpu():
             assert sect["frames"] == (4, 36) and sect["dec_color"][0] == 40 and sect["dec_color"][1] == _lib.lib().nsb_flat_decoder_floats(3)
             assert sect["grid_fine"][0] % 4 == 0 and total == sect["grid_fine"][0] + 320          # voxel sections are 16-byte aligned
             assert x.packed.numel() == 40 + ((15899 + 3) // 4) * 4 and x.d_frames.shape == (3, 12) and x.d_flat["color"].numel() == 15899
+
+
+def test_set_option_accepts_only_the_supported_decoder_backends():
+    """mlp_backend takes 0 (auto: tile kernels, FP32-FMA where S < 8) and 1 (FP32-FMA); other values and unknown keys are rejected."""
+    from nice_slam_b200 import _lib
+    L = _lib.lib()
+    NSB_ERR_ARG = -1
+    configured = int(os.environ.get("NSB_MLP_BACKEND", "0"))
+    try:
+        assert L.nsb_set_option(b"mlp_backend", 0) == 0
+        assert L.nsb_set_option(b"mlp_backend", 1) == 0
+        for value in (2, 3, -1):
+            assert L.nsb_set_option(b"mlp_backend", value) == NSB_ERR_ARG
+            assert b"mlp_backend" in L.nsb_last_error()
+        for key in (b"small_rays", b"pdl"):
+            assert L.nsb_set_option(key, 0) == NSB_ERR_ARG
+            assert b"unknown option" in L.nsb_last_error()
+    finally:
+        assert L.nsb_set_option(b"mlp_backend", configured) == 0

@@ -1,6 +1,6 @@
 #!/bin/bash
-# ncu evidence of the round: launch list of the bench command, full-set captures of the dominant kernels (ray-group kernels = default at 200 rays,
-# tile kernels, weight-gradient kernel).  Numbers printed under ncu are never bench values.
+# ncu evidence of the round: launch list of the bench command, full-set captures of the dominant kernels (tile kernels,
+# weight-gradient kernel).  Numbers printed under ncu are never bench values.
 tag=${1:-ev}
 mkdir -p gpurun_out
 export PYTHONUNBUFFERED=1

@@ -3,7 +3,7 @@ tag=${1:-q}
 mkdir -p gpurun_out
 export PYTHONUNBUFFERED=1
 timeout 900 python -m pytest tests -q -m gpu 2>&1 | tail -8 > gpurun_out/${tag}_tests.log; echo "pytest exit ${PIPESTATUS[0]}" >> gpurun_out/${tag}_tests.log; tail -4 gpurun_out/${tag}_tests.log
-for v in "NSB_X=0" "NSB_SMALL_RAYS=0"; do
+for v in "NSB_X=0"; do
   env $v NSB_BENCH_FAST=1 timeout 600 python bench.py --steps 300 --warmup 10 > gpurun_out/${tag}_fast_${v%%=*}.json 2>/dev/null
   python - <<PYEOF
 import json

@@ -22,8 +22,6 @@ for what in "$@"; do
       echo "bench exit $?"; tail -c 3000 gpurun_out/${tag}_bench.json; tail -5 gpurun_out/${tag}_bench.err ;;
     simt)
       NSB_MLP_BACKEND=1 timeout 900 python -m pytest tests -q -m gpu 2>&1 | tail -15 > gpurun_out/${tag}_tests_simt.log; tail -3 gpurun_out/${tag}_tests_simt.log ;;
-    old)
-      NSB_MLP_BACKEND=2 timeout 900 python -m pytest tests -q -m gpu 2>&1 | tail -15 > gpurun_out/${tag}_tests_old.log; tail -3 gpurun_out/${tag}_tests_old.log ;;
     ncu)
       timeout 900 ncu --metrics gpu__time_duration.sum --clock-control none -c 400 --csv --log-file gpurun_out/${tag}_launches.csv python bench.py --steps 2 --warmup 1 > gpurun_out/${tag}_ncu_bench.log 2>&1
       timeout 1200 ncu --set full --clock-control none --import-source on -k regex:render_.*tile -c 4 -o gpurun_out/${tag}_full python bench.py --steps 1 --warmup 1 > gpurun_out/${tag}_ncu_full.log 2>&1

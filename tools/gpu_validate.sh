@@ -4,8 +4,7 @@ mkdir -p gpurun_out
 export PYTHONUNBUFFERED=1
 timeout 600 python -m pytest tests/test_gpu_parity.py -q -m gpu -x -k "weight_gradients" 2>&1 | tail -30 > gpurun_out/${tag}_tests_wg.log; echo "pytest exit ${PIPESTATUS[0]}" >> gpurun_out/${tag}_tests_wg.log; tail -12 gpurun_out/${tag}_tests_wg.log
 timeout 900 python -m pytest tests -q -m gpu 2>&1 | tail -60 > gpurun_out/${tag}_tests.log; echo "pytest exit ${PIPESTATUS[0]}" >> gpurun_out/${tag}_tests.log; tail -8 gpurun_out/${tag}_tests.log
-NSB_SMALL_RAYS=0 timeout 900 python -m pytest tests -q -m gpu 2>&1 | tail -60 > gpurun_out/${tag}_tests_small0.log; echo "pytest exit ${PIPESTATUS[0]}" >> gpurun_out/${tag}_tests_small0.log; tail -4 gpurun_out/${tag}_tests_small0.log
-for v in "NSB_X=0" "NSB_SMALL_RAYS=0"; do
+for v in "NSB_X=0"; do
   env $v NSB_BENCH_FAST=1 timeout 600 python bench.py --steps 300 --warmup 10 > gpurun_out/${tag}_fast_${v%%=*}.json 2>/dev/null
   python - <<PYEOF
 import json

@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Cycle breakdown of one CTA of the tensor-core kernels (instrumented build: make -C nice_slam_b200/csrc ../libnsb_timing.so).
+"""Cycle breakdown of one CTA of the tile kernels (instrumented build: make -C nice_slam_b200/csrc ../libnsb_timing.so).
    NSB_LIB=nice_slam_b200/libnsb_timing.so python tools/phase_timing.py [n_rays]"""
 import ctypes as C
 import os
@@ -14,18 +14,12 @@ from gpu_util import make_renderer  # noqa: E402
 from nice_slam_b200 import _lib  # noqa: E402
 from nice_slam_b200.steps import IterationContext  # noqa: E402
 
-TILE_NAMES = {40: "fwd: launch -> depth max done", 41: "fwd: ray table (bbox far, near)", 42: "fwd: sample z", 43: "fwd: rank sort", 44: "fwd: point geometry + syncs",
-              1: "fwd: gather (per grid)", 2: "fwd: publish + issue fc_c", 6: "fwd: wait free buffer (E block)", 3: "fwd: embed block compute", 4: "fwd: publish + issue layer-0 block",
-              7: "fwd: wait MMAs of the layer", 8: "fwd: layer epilogue (tmem ld, relu, operand write)", 9: "fwd: publish + issue hidden layer", 12: "fwd: output layer + syncs",
-              14: "fwd: dealloc + sync", 15: "fwd: parts store + ray completion", 16: "fwd: compositing of completed rays",
-              20: "bwd: launch -> ray prologue (weights, dL/docc)", 21: "bwd: point geometry + sync", 22: "bwd: G/DU operand write", 23: "bwd: publish + issue layer", 24: "bwd: wait MMAs",
-              27: "bwd: dc rows + cos chain", 29: "bwd: scatter + dp", 30: "bwd: per-ray partial sums", 31: "bwd: ray completion", 32: "bwd: final ray reduce"}
-NAMES = {0: "fwd: tail sync of previous decoder", 1: "fwd: gather", 2: "fwd: fc_c publish + issue", 3: "fwd: E block 0", 4: "fwd: E block 1",
-         5: "fwd: E block 2", 6: "fwd: wait fc_c / layer-0 MMAs", 7: "fwd: layer step 0", 8: "fwd: layer step 1", 9: "fwd: layer step 2",
-         10: "fwd: layer step 3", 11: "fwd: layer 4 epilogue", 12: "fwd: output layer", 13: "fwd: sampling prologue", 14: "fwd: tmem dealloc",
-         15: "fwd: compositing + store", 20: "bwd: tail sync / scatter of previous decoder", 21: "bwd: header wait + g init", 22: "bwd: layer 4",
-         23: "bwd: layer 3", 24: "bwd: layer 2", 25: "bwd: layer 1", 26: "bwd: layer 0", 27: "bwd: dc rows + embedding chain", 28: "bwd: sync",
-         29: "bwd: scatter", 30: "bwd: ray reduce"}
+NAMES = {40: "fwd: launch -> depth max done", 41: "fwd: ray table (bbox far, near)", 42: "fwd: sample z", 43: "fwd: rank sort", 44: "fwd: point geometry + syncs",
+         1: "fwd: gather (per grid)", 2: "fwd: publish + issue fc_c", 6: "fwd: wait free buffer (E block)", 3: "fwd: embed block compute", 4: "fwd: publish + issue layer-0 block",
+         7: "fwd: wait MMAs of the layer", 8: "fwd: layer epilogue (tmem ld, relu, operand write)", 9: "fwd: publish + issue hidden layer", 12: "fwd: output layer + syncs",
+         14: "fwd: dealloc + sync", 15: "fwd: parts store + ray completion", 16: "fwd: compositing of completed rays",
+         20: "bwd: launch -> ray prologue (weights, dL/docc)", 21: "bwd: point geometry + sync", 22: "bwd: G/DU operand write", 23: "bwd: publish + issue layer", 24: "bwd: wait MMAs",
+         27: "bwd: dc rows + cos chain", 29: "bwd: scatter + dp", 30: "bwd: per-ray partial sums", 31: "bwd: ray completion", 32: "bwd: final ray reduce"}
 
 
 def main():
@@ -51,7 +45,7 @@ def main():
     for i in range(64):
         if buf[i]:
             tot = tot_f if i < 20 else tot_b
-            print("  %2d %-46s %9.0f  %5.1f %%" % (i, (TILE_NAMES if os.environ.get("NSB_MLP_BACKEND", "0") in ("0", "3") else NAMES).get(i, "?"), buf[i] / iters, 100.0 * buf[i] / tot))
+            print("  %2d %-46s %9.0f  %5.1f %%" % (i, NAMES.get(i, "?"), buf[i] / iters, 100.0 * buf[i] / tot))
 
 
 if __name__ == "__main__":
